@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the ray-marched NeRF step (BASELINE.json: train rays/s & render Msamples/s on a
 lego-shape 800x800 synthetic scene at 1/2/4/8 B200, % of roofline).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU, NCCL); training shards RAYS (4096 per GPU, weak scaling) with one
 exchange of the hash-grid + MLP gradients per step.  A "step" is one full training step of configs[1]:
@@ -20,6 +20,12 @@ Besides the headline (`value`, `e2e`, `roofline`, `cpu_baseline`) the line carri
 
 `--impl reference` times the CPU arm: the PyTorch-CPU restatement of the reference's non-cuda_ray renderer
 (oracle/cpu_renderer.py, BASELINE.json configs[0]) on the host cores, same metric and unit, exactly K timed steps.
+
+`--dump-outputs DIR` writes what the last of the K timed steps returned -- loss, image, depth (of the rays that enter the box),
+weights_sum, nears, num_points -- as DIR/<name>.npy.  Scenes, batches and initial weights are seeded, so two builds run with the
+same arguments can be compared output for output (up to the run-to-run order of the fp16 atomic gradient sums).  The step is the
+graph-replayed one that `value` times, so with the look-ahead pipeline (the default) the loss and per-ray results are those of
+the batch handed to the step before the last, and with N > 1 they are rank 0's shard of the rays.
 """
 from __future__ import annotations
 
@@ -344,9 +350,16 @@ def train_config(ctx, name, headline):
             gstep, graph_note = None, f"eager (graph capture failed: {type(e).__name__}: {e})"[:300]
             torch.cuda.synchronize()
     run = gstep if gstep is not None else (lambda *b: step(*b))
+    last = [None]
+
+    def timed_step(i):
+        last[0] = run(*dev_batches[i % nb])
+
     clocks = ClockSampler(ctx.local).start() if ctx.rank == 0 else None
-    ms = ctx.timed_loop(lambda i: run(*dev_batches[i % nb]), steps)
+    ms = ctx.timed_loop(timed_step, steps)
     clk = clocks.stop() if clocks else None
+    if headline and args.dump_outputs and ctx.rank == 0:
+        dump_outputs(args.dump_outputs, *last[0])
     graph_seen = model.step_counter[: min(16, steps), 0].tolist()
     graph_rows = int(gstep.out["num_points"]) if gstep is not None else rows
     dropped_samples += int(sum(max(0, c - graph_rows) for c in graph_seen))
@@ -486,6 +499,24 @@ def train_config(ctx, name, headline):
             res["value_with_occupancy_update"] = {"error": f"{type(e).__name__}: {e}"[:300]}
     res["_model"], res["_sc"], res["_step"], res["_batches"] = model, sc, step, (host_batches, dev_batches)
     return res
+
+
+def dump_outputs(out_dir, loss, out):
+    """What the last timed step returned to its caller -- the loss, the per-ray image / depth / weights_sum / nears and the sample
+    count -- as DIR/<name>.npy (float32; the count float64).  Called right after the timed loop: the later passes of the benchmark
+    replay the graph again, which overwrites these buffers.
+
+    `depth` holds the rays that enter the scene box only.  A ray that misses it has near == far == FLT_MAX (raymarching.cu:122), and
+    the depth normalisation of renderer.py:328 gives it 0 / 0 = NaN, a value that says nothing about the build; which rays miss is
+    fixed by the inputs and visible in `nears`."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = dict(out, loss=loss)
+    arrays["depth"] = out["depth"][out["nears"] < torch.finfo(torch.float32).max]
+    for name, v in arrays.items():
+        a = v.detach().float().cpu().numpy() if torch.is_tensor(v) else np.float64(v)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def count_real_samples(ctx, model, ro_d, rd_d):
@@ -882,7 +913,12 @@ def main():
     ap.add_argument("--no-gpu-ref", action="store_true", help="skip the gpu_reference leg")
     ap.add_argument("--no-configs", action="store_true", help="skip BASELINE configs 3-5")
     ap.add_argument("--no-large", action="store_true", help="skip the large-batch kernel roofline")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed training step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3)
 
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))

@@ -19,6 +19,38 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 
+MARCH_MILLION = [("lego", 1 << 20, 0.0), ("flower", 1 << 20, 0.0), ("bonsai", 1 << 20, 0.0), ("bonsai", 1 << 18, 1.0 / 256)]
+
+
+def march_million(out_dir):
+    """ref_march_million.json: digests of the reference's march_rays_train on the inputs of
+    tests/test_gpu_live_reference.py::test_march_train_counts_bit_exact_on_a_million_rays (its helpers, the reference kernel)."""
+    import torch
+    import ref_step
+    import test_gpu_live_reference as T
+    dev = torch.device("cuda", 0)
+    rm = ref_step.backend("_raymarching")
+    out = {}
+    for name, n, dt_gamma in MARCH_MILLION:
+        sc, ro, rd = T._all_rays(name, n, 11, dev)
+        n = ro.shape[0]
+        bits = torch.from_numpy(sc.density_bitfield).to(dev)
+        nears, fars = torch.empty(n, device=dev), torch.empty(n, device=dev)
+        rm.near_far_from_aabb(ro, rd, torch.from_numpy(sc.aabb).to(dev), n, float(sc.min_near), nears, fars)
+        noises = torch.rand(n, device=dev, generator=torch.Generator(device=dev).manual_seed(5))
+        _, _, _, rays, cnt = T._march_ref(rm, sc, ro, rd, bits, nears, fars, noises, 128, dt_gamma)
+        counts = rays[torch.argsort(rays[:, 0].long())][:, 2]
+        k = min(65536, n)
+        sub = [x[:k].contiguous() for x in (ro, rd, nears, fars, noises)]
+        xr, dr, lr, rr, c2 = T._march_ref(rm, sc, sub[0], sub[1], bits, sub[2], sub[3], sub[4], int(counts[:k].sum()) + 128, dt_gamma)
+        cnt_b, (xb, db, lb) = T._canonical(rr, xr, dr, lr)
+        out[f"{name}_{n}_{dt_gamma:g}"] = dict(near_far=T._digest(nears, fars), counter=cnt.tolist(), counts=T._digest(counts),
+                                               subset_counter=c2.tolist(), subset_counts=T._digest(cnt_b), subset_xyzs=T._digest(xb),
+                                               subset_dirs=T._digest(db), subset_deltas=T._digest(lb))
+    with open(os.path.join(out_dir, "ref_march_million.json"), "w") as f:
+        json.dump(out, f, indent=1)
+
+
 def main():
     import torch  # noqa: F401  (libtorch symbols must be loaded before the extension modules)
     from backends import OursBackend, RefBackend
@@ -26,7 +58,10 @@ def main():
 
     out_dir = os.path.join(ROOT, "gpurun_out", "golden")
     os.makedirs(out_dir, exist_ok=True)
-    want = sys.argv[1:] or list(CASES)
+    want = sys.argv[1:] or list(CASES) + ["march_million"]
+    if "march_million" in want:
+        march_million(out_dir)
+        want.remove("march_million")
     ref = RefBackend()
     ours = None
     try:

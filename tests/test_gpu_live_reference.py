@@ -13,6 +13,8 @@ names -- the parity holes VERDICT round 1 listed under "No oracle comparison at 
 Everything goes through the C ABI (ctypes) on our side and through the pybind11 modules on the reference side.
 """
 import ctypes as C
+import hashlib
+import json
 import os
 import sys
 
@@ -111,47 +113,112 @@ def _bits_equal(a, b):
     return bool(((a.view(torch.int32) == b.view(torch.int32)) | ((a == 0) & (b == 0))).all())
 
 
+def _digest(*tensors):
+    """sha256 of the bits of the tensors (floats with -0 folded into +0, which _bits_equal does not tell apart)."""
+    h = hashlib.sha256()
+    for t in tensors:
+        t = t + 0.0 if t.is_floating_point() else t
+        h.update(t.contiguous().cpu().numpy().tobytes())
+    return h.hexdigest()
+
+
+@pytest.fixture(scope="module")
+def march_golden():
+    with open(os.path.join(ROOT, "tests", "golden", "ref_march_million.json")) as f:
+        return json.load(f)
+
+
 @pytest.mark.parametrize("name,n,dt_gamma", [("lego", 1 << 20, 0.0), ("flower", 1 << 20, 0.0), ("bonsai", 1 << 20, 0.0),
                                              ("bonsai", 1 << 18, 1.0 / 256)])
-def test_march_train_counts_bit_exact_on_a_million_rays(dev, ref, name, n, dt_gamma):
+def test_march_train_counts_bit_exact_on_a_million_rays(dev, march_golden, name, n, dt_gamma):
+    """Against the reference's march_rays_train on the same rays, bit for bit.  The reference's results are stored as digests in
+    tests/golden/ref_march_million.json (near/far, per-ray counts of every ray, positions / directions / deltas of a 65 536-ray
+    subset, in ray-id order); where oracle/_ref is built the reference kernel is also run live."""
+    import ref_step
     sc, ro, rd = _all_rays(name, n, 11, dev)
     n = ro.shape[0]
     assert n >= 750_000 or dt_gamma > 0 or name == "flower"  # flower: 4 x 190 512 pixels exist in total
+    gold = march_golden[f"{name}_{n}_{dt_gamma:g}"]
+    rm = ref_step.backend("_raymarching") if ref_step.ref_available() else None
     bits = torch.from_numpy(sc.density_bitfield).to(dev)
     nears, fars = _near_far_ours(sc, ro, rd)
-    rn, rf = torch.empty_like(nears), torch.empty_like(fars)
-    ref["_raymarching"].near_far_from_aabb(ro, rd, torch.from_numpy(sc.aabb).to(dev), n, float(sc.min_near), rn, rf)
-    assert _bits_equal(nears, rn) and _bits_equal(fars, rf)
+    assert _digest(nears, fars) == gold["near_far"]
+    if rm is not None:
+        rn, rf = torch.empty_like(nears), torch.empty_like(fars)
+        rm.near_far_from_aabb(ro, rd, torch.from_numpy(sc.aabb).to(dev), n, float(sc.min_near), rn, rf)
+        assert _bits_equal(nears, rn) and _bits_equal(fars, rf)
     noises = torch.rand(n, device=dev, generator=torch.Generator(device=dev).manual_seed(5))
     # pass 1 with a token buffer: every ray overflows (nothing is written) but `rays` rows and the counters are complete
     _, _, _, rays_o_, cnt_o = _march_ours(sc, ro, rd, bits, nears, fars, noises, 128, dt_gamma)
-    _, _, _, rays_r_, cnt_r = _march_ref(ref["_raymarching"], sc, ro, rd, bits, nears, fars, noises, 128, dt_gamma)
-    assert cnt_o.tolist() == cnt_r.tolist() and cnt_o[1].item() == n
+    assert cnt_o.tolist() == gold["counter"] and cnt_o[1].item() == n
     co = rays_o_[torch.argsort(rays_o_[:, 0].long())][:, 2]
-    cr = rays_r_[torch.argsort(rays_r_[:, 0].long())][:, 2]
-    assert torch.equal(co, cr), f"{int((co != cr).sum())} of {n} per-ray sample counts differ"
+    assert _digest(co) == gold["counts"], "per-ray sample counts differ from the reference's"
+    if rm is not None:
+        _, _, _, rays_r_, cnt_r = _march_ref(rm, sc, ro, rd, bits, nears, fars, noises, 128, dt_gamma)
+        assert cnt_o.tolist() == cnt_r.tolist()
+        cr = rays_r_[torch.argsort(rays_r_[:, 0].long())][:, 2]
+        assert torch.equal(co, cr), f"{int((co != cr).sum())} of {n} per-ray sample counts differ"
     assert int(co.sum()) == int(cnt_o[0]) and int(co.max()) > 8
     # pass 2 on a 65 536-ray subset with room for every sample: positions, directions and deltas bit for bit
     k = min(65536, n)
     sro, srd, sn, sf, sno = ro[:k].contiguous(), rd[:k].contiguous(), nears[:k].contiguous(), fars[:k].contiguous(), noises[:k].contiguous()
     M = int(co[:k].sum()) + 128
     xo, do_, lo, ro_rows, c2 = _march_ours(sc, sro, srd, bits, sn, sf, sno, M, dt_gamma)
-    xr, dr, lr, rr_rows, c3 = _march_ref(ref["_raymarching"], sc, sro, srd, bits, sn, sf, sno, M, dt_gamma)
-    assert c2.tolist() == c3.tolist()
     total = int(c2[0])
     assert bool((xo[total:] == 0).all()) and bool((lo[total:] == 0).all())  # self-zeroed tail == torch.zeros + reference kernel
     cnt_a, (xa, da, la) = _canonical(ro_rows, xo, do_, lo)
-    cnt_b, (xb, db, lb) = _canonical(rr_rows, xr, dr, lr)
-    assert torch.equal(cnt_a, cnt_b)
-    assert _bits_equal(xa, xb) and _bits_equal(da, db) and _bits_equal(la, lb)
+    assert c2.tolist() == gold["subset_counter"] and _digest(cnt_a) == gold["subset_counts"]
+    assert _digest(xa) == gold["subset_xyzs"] and _digest(da) == gold["subset_dirs"] and _digest(la) == gold["subset_deltas"]
+    if rm is not None:
+        xr, dr, lr, rr_rows, c3 = _march_ref(rm, sc, sro, srd, bits, sn, sf, sno, M, dt_gamma)
+        assert c2.tolist() == c3.tolist()
+        cnt_b, (xb, db, lb) = _canonical(rr_rows, xr, dr, lr)
+        assert torch.equal(cnt_a, cnt_b)
+        assert _bits_equal(xa, xb) and _bits_equal(da, db) and _bits_equal(la, lb)
 
 
-def test_inference_rounds_bonsai_full_view_bit_exact(dev, ref):
+class _OracleRaymarching:
+    """march_rays / composite_rays of the CPU oracle (oracle/oracle.c, raymarching.cu restated; tests/test_oracle_golden.py holds it
+    to the reference's golden vectors bit for bit) behind the reference module's in-place signatures (raymarching/src/bindings.cpp)."""
+
+    def __init__(self):
+        from oracle import pyoracle
+        self.o = pyoracle
+
+    @staticmethod
+    def _h(t):
+        return t.cpu().numpy()
+
+    def march_rays(self, n_alive, n_step, alive, rays_t, ro, rd, bound, dt_gamma, max_steps, C, H, bits, nears, fars, xyzs, dirs, deltas,
+                   noises):
+        h = self._h
+        out = self.o.march_rays(n_alive, n_step, h(alive), h(rays_t), h(ro), h(rd), bound, h(bits), C, H, h(nears), h(fars), h(noises),
+                                xyzs.shape[0], dt_gamma, max_steps)
+        for dst, src in zip((xyzs, dirs, deltas), out):
+            dst.copy_(torch.from_numpy(src))
+
+    def composite_rays(self, n_alive, n_step, T_thresh, alive, rays_t, sigmas, rgbs, deltas, ws, depth, image):
+        h = self._h
+        out = self.o.composite_rays(n_alive, n_step, h(alive), h(rays_t), h(sigmas), h(rgbs), h(deltas), h(ws), h(depth), h(image),
+                                    T_thresh)
+        for dst, src in zip((alive, rays_t, ws, depth, image), out):
+            dst.copy_(torch.from_numpy(src))
+
+
+@pytest.fixture(scope="module")
+def raymarching_ref():
+    """The reference's raymarching extension where oracle/_ref is built, else the CPU oracle that restates it."""
+    import ref_step
+    return ref_step.backend("_raymarching") if ref_step.ref_available() else _OracleRaymarching()
+
+
+def test_inference_rounds_bonsai_full_view_bit_exact(dev, raymarching_ref):
     """The loop of run_cuda (renderer.py:335-387) on a full bonsai-shape view (bound 16, C = 5): in every round the SAME state
     (rays_alive, rays_t) goes through the reference's march_rays and ours, then through both compositors with synthetic
-    densities; the reference's results carry the state forward.  Positions / deltas bit-exact, kill pattern exact."""
+    densities; the reference's results carry the state forward.  Positions / deltas bit-exact, kill pattern exact.  Without
+    oracle/_ref the reference side is the CPU oracle's restatement of the same two kernels."""
     from laenerf_b200.scene import get_rays_np
-    N, rm = _N(), ref["_raymarching"]
+    N, rm = _N(), raymarching_ref
     sc = scene("bonsai")
     ro, rd, _ = get_rays_np(sc.poses[1], sc.intrinsics, sc.H, sc.W)
     ro, rd = torch.from_numpy(ro).to(dev), torch.from_numpy(rd).to(dev)
