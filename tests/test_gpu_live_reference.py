@@ -11,6 +11,9 @@ names -- the parity holes VERDICT round 1 listed under "No oracle comparison at 
   * lnrf_nerf_backward (the dominant call of the step) against the CPU oracle's composition of network_ff.py:51-79.
 
 Everything goes through the C ABI (ctypes) on our side and through the pybind11 modules on the reference side.
+
+The grid encoder is also checked without the reference: tests/test_gpu_grid_encoder.py compares every kernel path (the training
+shape of lego, flower and bonsai included) entry by entry with the CPU oracle, under tolerances derived from the arithmetic.
 """
 import ctypes as C
 import hashlib
