@@ -502,6 +502,21 @@ LNRF_API int lnrf_adam_step_sharded(const void* const* grad_peers_host, void* co
                                     double beta1, double beta2, double eps, double weight_decay, const float* grad_scale,
                                     float* found_inf_out, const float* step_count, const float* lr_scale,
                                     lnrf_stream_t stream);
+/* fp32 form of lnrf_adam_step_sharded for a network trained without fp16 shadows (the edit-stage style network): grad_peers /
+ * param_peers / flag_peers = HOST arrays of `world` pointers to each rank's full fp32 gradient vector, full fp32 parameter vector
+ * and non-finite flag.  This rank (`rank`) owns elements [lo, lo + n): it averages the `world` gradients of that slice in the fixed
+ * rank order 0 .. world-1 (every rank forms the same bits), unscales by *grad_scale, applies Adam with its fp32 moment slices and
+ * stores the new value into every rank's parameter vector -- the parameter vector is the master, no separate copy exists.
+ * Learning rate per part of the vector: n_segs (1..8) segments, segment s covers [seg_start[s], seg_start[s+1]) at
+ * lr x seg_lr_mult[s]; seg_start (HOST, elements of the full vector) begins at 0, ascends strictly and holds multiples of 8.
+ * Skip-on-inf and the caller's synchronisation as for lnrf_adam_step_sharded. */
+LNRF_API int lnrf_adam_step_sharded_f32(const float* const* grad_peers_host, float* const* param_peers_host,
+                                        const float* const* flag_peers_host, uint32_t world, uint32_t rank, uint64_t lo,
+                                        uint64_t n, const uint64_t* seg_start_host, const double* seg_lr_mult_host,
+                                        uint32_t n_segs, float* exp_avg_shard, float* exp_avg_sq_shard, double lr,
+                                        double beta1, double beta2, double eps, double weight_decay, const float* grad_scale,
+                                        float* found_inf_out, const float* step_count, const float* lr_scale,
+                                        lnrf_stream_t stream);
 /* The same for a loop that alternates TWO gradient buffers (and two flag words) between consecutive steps: while the ranks read this
  * step's buffer, the kernel clears the buffer the previous step used (other_grad_f16, other_n elements; its readers passed this step's
  * opening barrier long ago), zeroes that step's flag word (other_flag), and performs GradScaler.update() on the live words at its end.

@@ -90,6 +90,7 @@ SIGNATURES = {
     "lnrf_grad_nonfinite_check": (i32, [vp, u32, vp, vp]),
     "lnrf_adam_step": (i32, [vp, u32, f64, f64, f64, f64, f64, vp, vp, vp, vp, vp]),
     "lnrf_adam_step_sharded": (i32, [vp, vp, vp, u32, u64, u64, vp, vp, vp, f64, f64, f64, f64, f64, vp, vp, vp, vp, vp]),
+    "lnrf_adam_step_sharded_f32": (i32, [vp, vp, vp, u32, u32, u64, u64, vp, vp, u32, vp, vp, f64, f64, f64, f64, f64, vp, vp, vp, vp, vp]),
     "lnrf_adam_step_sharded_pipelined": (i32, [vp, vp, vp, u32, u64, u64, vp, vp, vp, f64, f64, f64, f64, f64, vp, vp, vp, u64, vp, vp, vp, vp, vp,
                                                f32, f32, i32, vp]),
     "lnrf_grad_nonfinite_check_snapshot": (i32, [vp, u32, vp, vp, vp, vp, vp]),

@@ -12,6 +12,8 @@
 // CUDA Adam arithmetic, including its double-precision intermediate steps), writes the fp16 shadow copy the next
 // forward gathers from, and clears the gradient: g16 R+W, p32 R+W, m R+W, v R+W, p16 W = 367 MB -- HBM-bound.
 // Several tensors (table + both MLP weight vectors) are served by the same two launches.
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace lnrf {
@@ -479,11 +481,50 @@ k_adam_amp_fused(const OptBatch b, AdamHyper h, const float* __restrict__ lr_sca
 // Synchronisation is the caller's: a cross-rank barrier before (gradients + flags complete) and after (shadows written,
 // gradients may be cleared) the launch.
 constexpr int kMaxPeers = 8;   // one NVSwitch domain of 8 GPUs; also bounds the registers that hold the in-flight peer loads
+// G = gradient element type, P = element type of the replicated vector the kernel stores into: (__half, __half) for the NeRF's fp16
+// gradients and fp16 shadow tables, (float, float) for the style network, whose fp32 parameter vector is both master and replica
+template <typename G, typename P>
 struct PeerPtrs {
-    const __half* grad[kMaxPeers];
-    __half* shadow[kMaxPeers];
+    const G* grad[kMaxPeers];
+    P* param[kMaxPeers];
     const float* flag[kMaxPeers];
 };
+// Per-segment learning rates of the flat vector (the style network trains its palette at 2 x lr): element e belongs to the last
+// segment whose start <= e.  Starts are multiples of 8 elements, so one thread's 8-element vector never straddles two segments.
+constexpr int kMaxLrSegments = 8;
+struct LrSegments {
+    uint64_t start[kMaxLrSegments];
+    double mult[kMaxLrSegments];
+    uint32_t count;
+};
+struct NoLrSegments {};
+// the step size of every segment, formed as adam_step_consts forms it for lr x mult (shared memory of the block)
+__device__ __forceinline__ float* segment_step_sizes(const AdamHyper& h, const LrSegments& segs, const float* step_count) {
+    __shared__ float s_step_size[kMaxLrSegments];
+    if (threadIdx.x < segs.count) {
+        const float bc1 = (float)(1.0 - pow(h.beta1, (double)*step_count));
+        s_step_size[threadIdx.x] = (float)(h.lr * segs.mult[threadIdx.x] / (double)bc1);
+    }
+    __syncthreads();
+    return s_step_size;
+}
+
+// eight consecutive gradient elements of one rank, loaded as 16-byte vectors and added to g[0..7] in fp32
+__device__ __forceinline__ uint4 ld_grad8(const __half* p) { return *reinterpret_cast<const uint4*>(p); }
+__device__ __forceinline__ void add_grad8(float* g, const uint4& u) {
+    union { uint4 u; __half2 h2[4]; } w;
+    w.u = u;
+#pragma unroll
+    for (int j = 0; j < 4; j++) { const float2 f = __half22float2(w.h2[j]); g[2 * j] += f.x; g[2 * j + 1] += f.y; }
+}
+struct Float8 { float4 a, b; };
+__device__ __forceinline__ Float8 ld_grad8(const float* p) {
+    return Float8{reinterpret_cast<const float4*>(p)[0], reinterpret_cast<const float4*>(p)[1]};
+}
+__device__ __forceinline__ void add_grad8(float* g, const Float8& u) {
+    g[0] += u.a.x; g[1] += u.a.y; g[2] += u.a.z; g[3] += u.a.w;
+    g[4] += u.b.x; g[5] += u.b.y; g[6] += u.b.z; g[7] += u.b.w;
+}
 
 // In-kernel rank synchronisation (ExchangeSync.epoch != nullptr).  The flag buffer of every rank is peer-mapped; words
 // [kSyncArrive + r] and [kSyncDone + r] of MY buffer are written by rank r only.  Epoch e = *epoch + 1 of this step:
@@ -530,11 +571,16 @@ __device__ __forceinline__ void wait_words_ge(const uint32_t* words, uint32_t R,
     __syncthreads();
 }
 
+// fp32 form (G = P = float): `master` is this rank's slice of its own parameter vector, which the broadcast store rewrites like every
+// other rank's; `segs` gives the learning rate of each part of the vector.
+template <typename G, typename P, typename Segs>
 __global__ void __launch_bounds__(kOptBlock)
-k_adam_step_p2p(const PeerPtrs peers, const uint32_t R, const uint64_t lo, const uint64_t n, float* __restrict__ master,
+k_adam_step_p2p(const PeerPtrs<G, P> peers, const uint32_t R, const uint64_t lo, const uint64_t n, float* __restrict__ master,
                 float* __restrict__ exp_avg, float* __restrict__ exp_avg_sq, AdamHyper h, const float* __restrict__ grad_scale,
                 float* __restrict__ found_inf_out, const float* __restrict__ step_count, const float* __restrict__ lr_scale,
-                const ExchangeSync sync, const ExchangeExtra extra) {
+                const ExchangeSync sync, const ExchangeExtra extra, const Segs segs) {
+    constexpr bool kF32 = std::is_same<P, float>::value;
+    static_assert(kF32 == std::is_same<Segs, LrSegments>::value, "segment table: fp32 form only");
     uint32_t epoch = 0;
     if (sync.epoch) {
         epoch = *sync.epoch + 1u;
@@ -552,20 +598,28 @@ k_adam_step_p2p(const PeerPtrs peers, const uint32_t R, const uint64_t lo, const
     if (blockIdx.x == 0 && threadIdx.x == 0) *found_inf_out = skip ? 1.0f : 0.0f;
     // GradScaler: when any rank saw a non-finite gradient nothing is updated (the gradients are cleared after the closing sync)
     if (lr_scale) h.lr *= (double)*lr_scale;
-    const AdamStepConsts c = adam_step_consts(h, grad_scale, step_count);
+    AdamStepConsts c = adam_step_consts(h, grad_scale, step_count);
     const float inv_R = 1.0f / (float)R;
+    float* s_step_size = nullptr;
+    if constexpr (kF32) s_step_size = segment_step_sizes(h, segs, step_count);
 
     for (uint64_t base = (uint64_t)blockIdx.x * kOptChunk; base < n && !skip; base += (uint64_t)gridDim.x * kOptChunk) {
         const uint64_t i = base + (uint64_t)threadIdx.x * kOptPerThread;  // n is a multiple of 8: no ragged tail
         if (i >= n) continue;
+        if constexpr (kF32) {
+            uint32_t k = 0;
+            for (uint32_t s = 1; s < segs.count; s++)
+                if (lo + i >= segs.start[s]) k = s;
+            c.step_size = s_step_size[k];
+        }
         float g[kOptPerThread], p[kOptPerThread], m[kOptPerThread], v[kOptPerThread];
 #pragma unroll
         for (int j = 0; j < (int)kOptPerThread; j++) g[j] = 0.0f;
         // all loads first: R gradient vectors (R-1 of them remote) + the local fp32 state
-        uint4 gw[kMaxPeers];
+        std::conditional_t<kF32, Float8, uint4> gw[kMaxPeers];
 #pragma unroll
         for (int r = 0; r < kMaxPeers; r++)
-            if (r < (int)R) gw[r] = *reinterpret_cast<const uint4*>(peers.grad[r] + lo + i);
+            if (r < (int)R) gw[r] = ld_grad8(peers.grad[r] + lo + i);
         *reinterpret_cast<float4*>(p) = *reinterpret_cast<const float4*>(master + i);
         *reinterpret_cast<float4*>(p + 4) = *reinterpret_cast<const float4*>(master + i + 4);
         *reinterpret_cast<float4*>(m) = *reinterpret_cast<const float4*>(exp_avg + i);
@@ -573,28 +627,34 @@ k_adam_step_p2p(const PeerPtrs peers, const uint32_t R, const uint64_t lo, const
         *reinterpret_cast<float4*>(v) = *reinterpret_cast<const float4*>(exp_avg_sq + i);
         *reinterpret_cast<float4*>(v + 4) = *reinterpret_cast<const float4*>(exp_avg_sq + i + 4);
 #pragma unroll
-        for (int r = 0; r < kMaxPeers; r++) {
-            if (r < (int)R) {
-                union { uint4 u; __half2 h2[4]; } w;
-                w.u = gw[r];
-#pragma unroll
-                for (int j = 0; j < 4; j++) { const float2 f = __half22float2(w.h2[j]); g[2 * j] += f.x; g[2 * j + 1] += f.y; }
-            }
-        }
+        for (int r = 0; r < kMaxPeers; r++)   // fixed rank order 0 .. R-1: every rank forms the same sum
+            if (r < (int)R) add_grad8(g, gw[r]);
 #pragma unroll
         for (int j = 0; j < (int)kOptPerThread; j++) adam_update(p[j], m[j], v[j], adam_unscale(g[j] * inv_R, c), h, c);
-        *reinterpret_cast<float4*>(master + i) = *reinterpret_cast<const float4*>(p);
-        *reinterpret_cast<float4*>(master + i + 4) = *reinterpret_cast<const float4*>(p + 4);
+        if constexpr (!kF32) {
+            *reinterpret_cast<float4*>(master + i) = *reinterpret_cast<const float4*>(p);
+            *reinterpret_cast<float4*>(master + i + 4) = *reinterpret_cast<const float4*>(p + 4);
+        }
         *reinterpret_cast<float4*>(exp_avg + i) = *reinterpret_cast<const float4*>(m);
         *reinterpret_cast<float4*>(exp_avg + i + 4) = *reinterpret_cast<const float4*>(m + 4);
         *reinterpret_cast<float4*>(exp_avg_sq + i) = *reinterpret_cast<const float4*>(v);
         *reinterpret_cast<float4*>(exp_avg_sq + i + 4) = *reinterpret_cast<const float4*>(v + 4);
-        union { uint4 u; __half2 h2[4]; } o;
+        if constexpr (kF32) {  // the broadcast IS the update: rank `me`'s own vector is one of the R
 #pragma unroll
-        for (int j = 0; j < 4; j++) o.h2[j] = __floats2half2_rn(p[2 * j], p[2 * j + 1]);
+            for (int r = 0; r < kMaxPeers; r++) {
+                if (r < (int)R) {
+                    reinterpret_cast<float4*>(peers.param[r] + lo + i)[0] = *reinterpret_cast<const float4*>(p);
+                    reinterpret_cast<float4*>(peers.param[r] + lo + i)[1] = *reinterpret_cast<const float4*>(p + 4);
+                }
+            }
+        } else {
+            union { uint4 u; __half2 h2[4]; } o;
 #pragma unroll
-        for (int r = 0; r < kMaxPeers; r++)
-            if (r < (int)R) *reinterpret_cast<uint4*>(peers.shadow[r] + lo + i) = o.u;
+            for (int j = 0; j < 4; j++) o.h2[j] = __floats2half2_rn(p[2 * j], p[2 * j + 1]);
+#pragma unroll
+            for (int r = 0; r < kMaxPeers; r++)
+                if (r < (int)R) *reinterpret_cast<uint4*>(peers.param[r] + lo + i) = o.u;
+        }
     }
     if (extra.clear) {
         for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < extra.clear_nvec; i += (uint64_t)gridDim.x * blockDim.x)
@@ -805,18 +865,19 @@ static int adam_step_sharded_impl(const void* const* grad_peers_host, void* cons
                  "adam_step_sharded: null pointer");
     LNRF_REQUIRE(n % 8 == 0 && lo % 8 == 0, "adam_step_sharded: slice offset / length must be multiples of 8 elements");
     if (n == 0) return LNRF_OK;
-    PeerPtrs pp{};
+    PeerPtrs<__half, __half> pp{};
     for (uint32_t r = 0; r < world; r++) {
         LNRF_REQUIRE(grad_peers_host[r] && shadow_peers_host[r] && flag_peers_host[r], "adam_step_sharded: null peer pointer (rank %u)", r);
         pp.grad[r] = (const __half*)grad_peers_host[r];
-        pp.shadow[r] = (__half*)shadow_peers_host[r];
+        pp.param[r] = (__half*)shadow_peers_host[r];
         pp.flag[r] = flag_peers_host[r];
     }
     AdamHyper h{lr, beta1, beta2, eps, weight_decay};
     const uint64_t chunks = (n + kOptChunk - 1) / kOptChunk, cap = (uint64_t)kNumSMs * 8;
     ExchangeSync sy{sync_epoch, sync_ticket, rank};
-    k_adam_step_p2p<<<(uint32_t)(chunks < cap ? chunks : cap), kOptBlock, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-        pp, world, lo, n, master_shard, exp_avg_shard, exp_avg_sq_shard, h, grad_scale, found_inf_out, step_count, lr_scale, sy, extra);
+    k_adam_step_p2p<__half, __half, NoLrSegments><<<(uint32_t)(chunks < cap ? chunks : cap), kOptBlock, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+        pp, world, lo, n, master_shard, exp_avg_shard, exp_avg_sq_shard, h, grad_scale, found_inf_out, step_count, lr_scale, sy, extra,
+        NoLrSegments{});
     LNRF_LAUNCH_CHECK("adam_step_sharded");
     return LNRF_OK;
 }
@@ -839,6 +900,48 @@ int lnrf_adam_step_sharded_sync(const void* const* grad_peers_host, void* const*
     return adam_step_sharded_impl(grad_peers_host, shadow_peers_host, flag_peers_host, world, lo, n, master_shard, exp_avg_shard,
                                   exp_avg_sq_shard, lr, beta1, beta2, eps, weight_decay, grad_scale, found_inf_out, step_count, lr_scale, rank,
                                   sync_state, sync_state + 1, stream);
+}
+
+int lnrf_adam_step_sharded_f32(const float* const* grad_peers_host, float* const* param_peers_host, const float* const* flag_peers_host,
+                               uint32_t world, uint32_t rank, uint64_t lo, uint64_t n, const uint64_t* seg_start_host,
+                               const double* seg_lr_mult_host, uint32_t n_segs, float* exp_avg_shard, float* exp_avg_sq_shard, double lr,
+                               double beta1, double beta2, double eps, double weight_decay, const float* grad_scale, float* found_inf_out,
+                               const float* step_count, const float* lr_scale, lnrf_stream_t stream) {
+    LNRF_REQUIRE(world >= 1 && world <= (uint32_t)kMaxPeers, "adam_step_sharded_f32: 1..%d ranks, got %u", kMaxPeers, world);
+    LNRF_REQUIRE(rank < world, "adam_step_sharded_f32: rank %u outside the world of %u", rank, world);
+    LNRF_REQUIRE(grad_peers_host && param_peers_host && flag_peers_host && seg_start_host && seg_lr_mult_host && exp_avg_shard &&
+                     exp_avg_sq_shard && found_inf_out && step_count,
+                 "adam_step_sharded_f32: null pointer");
+    LNRF_REQUIRE(n % 8 == 0 && lo % 8 == 0, "adam_step_sharded_f32: slice offset / length must be multiples of 8 elements");
+    LNRF_REQUIRE(n_segs >= 1 && n_segs <= (uint32_t)kMaxLrSegments, "adam_step_sharded_f32: 1..%d lr segments, got %u", kMaxLrSegments, n_segs);
+    LrSegments segs{};
+    segs.count = n_segs;
+    for (uint32_t s = 0; s < n_segs; s++) {
+        LNRF_REQUIRE(s == 0 ? seg_start_host[0] == 0 : seg_start_host[s] > seg_start_host[s - 1],
+                     "adam_step_sharded_f32: segment starts must begin at 0 and ascend strictly (segment %u)", s);
+        LNRF_REQUIRE(seg_start_host[s] % 8 == 0, "adam_step_sharded_f32: segment %u starts off a multiple of 8 elements", s);
+        LNRF_REQUIRE(seg_lr_mult_host[s] >= 0.0 && seg_lr_mult_host[s] < 1e30, "adam_step_sharded_f32: segment %u: bad lr multiplier", s);
+        segs.start[s] = seg_start_host[s];
+        segs.mult[s] = seg_lr_mult_host[s];
+    }
+    PeerPtrs<float, float> pp{};
+    uintptr_t align = reinterpret_cast<uintptr_t>(exp_avg_shard) | reinterpret_cast<uintptr_t>(exp_avg_sq_shard);
+    for (uint32_t r = 0; r < world; r++) {
+        LNRF_REQUIRE(grad_peers_host[r] && param_peers_host[r] && flag_peers_host[r], "adam_step_sharded_f32: null peer pointer (rank %u)", r);
+        pp.grad[r] = grad_peers_host[r];
+        pp.param[r] = param_peers_host[r];
+        pp.flag[r] = flag_peers_host[r];
+        align |= reinterpret_cast<uintptr_t>(grad_peers_host[r]) | reinterpret_cast<uintptr_t>(param_peers_host[r]);
+    }
+    LNRF_REQUIRE((align & 15) == 0, "adam_step_sharded_f32: buffers must be 16-byte aligned");
+    if (n == 0) return LNRF_OK;
+    AdamHyper h{lr, beta1, beta2, eps, weight_decay};
+    const uint64_t chunks = (n + kOptChunk - 1) / kOptChunk, cap = (uint64_t)kNumSMs * 8;
+    k_adam_step_p2p<float, float, LrSegments><<<(uint32_t)(chunks < cap ? chunks : cap), kOptBlock, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+        pp, world, lo, n, param_peers_host[rank] + lo, exp_avg_shard, exp_avg_sq_shard, h, grad_scale, found_inf_out, step_count, lr_scale,
+        ExchangeSync{nullptr, nullptr, rank}, ExchangeExtra{}, segs);
+    LNRF_LAUNCH_CHECK("adam_step_sharded_f32");
+    return LNRF_OK;
 }
 
 int lnrf_adam_step_sharded_pipelined(const void* const* grad_peers_host, void* const* shadow_peers_host, const float* const* flag_peers_host,

@@ -53,7 +53,7 @@ class _grid_encode(Function):
     @staticmethod
     @custom_fwd(device_type="cuda")
     def forward(ctx, inputs, embeddings, offsets, per_level_scale, base_resolution, calc_grad_inputs=False, gridtype=0,
-                align_corners=False, interpolation=0, shadow_f16=None, grad_f16=None, world_bound=0.0, b_dev=None):
+                align_corners=False, interpolation=0, shadow_f16=None, grad_f16=None, world_bound=0.0, b_dev=None, grad_f32=None):
         # b_dev: optional device int32 with the number of live rows (world_bound > 0 only): whole 128-row tiles past it are neither
         # encoded nor differentiated -- their output rows stay unwritten, which is fine for a consumer that honours the same count
         # world_bound > 0: `inputs` are world coordinates and the kernel applies GridEncoder.forward's (x + bound) / (2 * bound)
@@ -64,13 +64,15 @@ class _grid_encode(Function):
         C = embeddings.shape[1]
         S = float(np.log2(per_level_scale))
         H = int(base_resolution)
-        ctx.grad_f16 = None
+        ctx.grad_buf = None
         if torch.is_autocast_enabled() and C % 2 == 0:  # grid.py:43-44
             if shadow_f16 is not None:  # laenerf_b200.optim.AmpAdam keeps embeddings.half() up to date: no cast pass
                 embeddings = shadow_f16
-                ctx.grad_f16 = grad_f16
+                ctx.grad_buf = grad_f16
             else:
                 embeddings = embeddings.to(torch.half)
+        elif grad_f32 is not None and embeddings.dtype == torch.float32:
+            ctx.grad_buf = grad_f32  # the fp32 table read directly (no autocast) with a persistent fp32 gradient buffer
         embeddings = embeddings.contiguous()
         off_h = _offsets_host(offsets)
         outputs = torch.empty(B, L * C, device=inputs.device, dtype=embeddings.dtype)
@@ -99,8 +101,9 @@ class _grid_encode(Function):
         inputs, embeddings, offsets, dy_dx, b_dev = ctx.saved_tensors
         B, D, C, L, S, H, gridtype, interpolation = ctx.dims
         grad = grad.contiguous().to(embeddings.dtype)
-        # with AmpAdam the gradient accumulates straight into its persistent fp16 buffer (cleared by the optimizer kernel)
-        grad_embeddings = ctx.grad_f16 if ctx.grad_f16 is not None else torch.zeros_like(embeddings)
+        # with AmpAdam the gradient accumulates straight into its persistent fp16 buffer (cleared by the optimizer kernel); with
+        # ShardedFlatAdam into this rank's fp32 gradient vector, which the other ranks read over NVLink
+        grad_embeddings = ctx.grad_buf if ctx.grad_buf is not None else torch.zeros_like(embeddings)
         grad_inputs = torch.zeros_like(inputs, dtype=embeddings.dtype) if dy_dx is not None else None
         if ctx.world_bound > 0:
             N.check(N.lib().lnrf_grid_encode_backward_world(N.ptr(grad), N.ptr(inputs), ctx.world_bound, N.ptr(_offsets_host(offsets)),
@@ -113,9 +116,9 @@ class _grid_encode(Function):
                                                       _dt(embeddings), N.GRID_BLC, N.stream()))
         if dy_dx is not None:
             grad_inputs = grad_inputs.to(inputs.dtype)
-        if ctx.grad_f16 is not None:
+        if ctx.grad_buf is not None:
             grad_embeddings = None
-        return grad_inputs, grad_embeddings, None, None, None, None, None, None, None, None, None, None, None
+        return grad_inputs, grad_embeddings, None, None, None, None, None, None, None, None, None, None, None, None
 
 
 grid_encode = _grid_encode.apply
@@ -157,6 +160,8 @@ class GridEncoder(nn.Module):
         # set by laenerf_b200.optim.AmpAdam: fp16 shadow of the table + persistent fp16 gradient (row f-4)
         self._shadow_f16 = None
         self._grad_f16 = None
+        # set by laenerf_b200.optim.ShardedFlatAdam: persistent fp32 gradient of the fp32 table, used when no autocast casts it
+        self._grad_f32 = None
 
     def reset_parameters(self):
         std = 1e-4
@@ -180,7 +185,8 @@ class GridEncoder(nn.Module):
         inputs = inputs.view(-1, self.input_dim)
         outputs = grid_encode(inputs, self.embeddings, self.offsets, self.per_level_scale, self.base_resolution,
                               inputs.requires_grad, self.gridtype_id, self.align_corners, self.interp_id,
-                              shadow_f16(self, self.embeddings), self._grad_f16, float(bound) if in_kernel else 0.0, b_dev)
+                              shadow_f16(self, self.embeddings), self._grad_f16, float(bound) if in_kernel else 0.0, b_dev,
+                              self._grad_f32)
         return outputs.view(prefix_shape + [self.output_dim])
 
     @torch.autocast(device_type="cuda", enabled=False)

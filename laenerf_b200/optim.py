@@ -569,3 +569,184 @@ class AmpAdam:
         if "scaler" in sd:  # round-1 checkpoints nested the scaler state here
             self.load_scaler_state_dict(sd["scaler"])
         self._resync_if_params_changed()
+
+
+class ShardedFlatAdam(AmpAdam):
+    """Data-parallel Adam + GradScaler for a network trained in fp32 without fp16 shadows (the edit-stage style network, row a-13),
+    sharded ZeRO-1 style over torch symmetric memory.
+
+    The parameters of all owners are views of ONE flat fp32 vector (each tensor starts on a multiple of 8 elements, the vector is
+    padded to a multiple of 8 x world), peer-mapped on every rank; so is the flat fp32 gradient vector.  Owners with `persistent` set
+    accumulate into it from their kernels (GridEncoder's `_grad_f32`: the 49 MB table gradient is never copied); the gradients of the
+    others arrive through autograd and are copied into their place by step() (the two small nets and the palette: ~10 K values).
+    step() = inf check of the local gradient (flag published beside it) -> barrier -> ONE kernel (lnrf_adam_step_sharded_f32): this
+    rank averages the R gradients of its slice in rank order, runs Adam on it with per-owner learning rates and stores the new values
+    into every rank's parameter vector -> barrier -> gradient clear + GradScaler.update().  Adam moments exist for the slice only.
+    No host synchronisation, so the step can be captured in a CUDA graph.
+
+    world_size = 1 needs no process group: the vectors are ordinary device memory and the only peer is the rank itself.  Construction
+    raises when the symmetric-memory rendezvous fails; nothing has been re-pointed then."""
+
+    def __init__(self, owners, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, init_scale=2.0 ** 16, growth_factor=2.0,
+                 backoff_factor=0.5, growth_interval=2000, world_size=1, rank=0, group=None, n_groups=None):
+        self.model = None
+        self.lr, self.betas, self.eps, self.weight_decay = float(lr), (float(betas[0]), float(betas[1])), float(eps), float(weight_decay)
+        self.fp16, self.sharded = True, False
+        self.growth_factor, self.backoff_factor, self.growth_interval = float(growth_factor), float(backoff_factor), int(growth_interval)
+        self.world, self.rank, self.group = int(world_size), int(rank), group
+        self.owners = [o if isinstance(o, _Owner) else _Owner(*o) for o in owners]
+        self.n_groups = int(n_groups) if n_groups is not None else 1 + max(o.group for o in self.owners)
+        dev = self.owners[0].param.device
+        if dev.type != "cuda":
+            raise RuntimeError("ShardedFlatAdam: the parameters must live on a CUDA device (there is no CPU path)")
+        if any(o.param.dtype != torch.float32 for o in self.owners):
+            raise RuntimeError("ShardedFlatAdam: fp32 parameters only")
+        self._offsets, off = [], 0
+        for o in self.owners:
+            self._offsets.append(off)
+            off += (o.param.numel() + 7) // 8 * 8
+        unit = 8 * self.world
+        self.P_pad = (off + unit - 1) // unit * unit
+        self.Sz = self.P_pad // self.world
+        self.lo, self.hi = self.rank * self.Sz, (self.rank + 1) * self.Sz
+        # learning-rate segments: runs of owners with the same multiplier
+        starts, mults = [], []
+        for o, o_off in zip(self.owners, self._offsets):
+            if not mults or mults[-1] != o.lr_mult:
+                starts.append(o_off)
+                mults.append(o.lr_mult)
+        if len(starts) > 8:
+            raise RuntimeError("ShardedFlatAdam: at most 8 learning-rate segments")
+        self._seg_start, self._seg_mult = (C.c_uint64 * len(starts))(*starts), (C.c_double * len(mults))(*mults)
+        self.p2p = None
+        if self.world > 1:
+            self._init_symmetric(dev)
+        else:
+            self.param_flat = torch.zeros(self.P_pad, dtype=torch.float32, device=dev)
+            self.grad_flat = torch.zeros(self.P_pad, dtype=torch.float32, device=dev)
+            self.flag_buf = torch.zeros(32, dtype=torch.float32, device=dev)
+            self._peer_arrays = tuple((C.c_void_p * 1)(t.data_ptr()) for t in (self.grad_flat, self.param_flat, self.flag_buf))
+        # re-point every parameter into the flat vector (a leaf stays the same leaf: the palette is a plain tensor, not an nn.Parameter)
+        self._grad_views = []
+        with torch.no_grad():
+            for o, o_off in zip(self.owners, self._offsets):
+                n = o.param.numel()
+                view = self.param_flat[o_off:o_off + n].view_as(o.param)
+                view.copy_(o.param)
+                o.param.set_(view)
+                gview = self.grad_flat[o_off:o_off + n].view_as(o.param)
+                self._grad_views.append(gview)
+                if o.persistent:
+                    o.module._grad_f32 = gview
+        if self.world > 1:
+            torch.cuda.synchronize()
+            self.p2p["grad"].barrier(channel=0)
+        self.state = [{"exp_avg": torch.zeros(self.Sz, dtype=torch.float32, device=dev),
+                       "exp_avg_sq": torch.zeros(self.Sz, dtype=torch.float32, device=dev)}]
+        self.step_count = torch.ones(1, dtype=torch.float32, device=dev)
+        self.found_inf = torch.zeros(1, dtype=torch.float32, device=dev)
+        self._scale = torch.full((1,), float(init_scale), dtype=torch.float32, device=dev)
+        self._growth_tracker = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.lr_scale = torch.ones(1, dtype=torch.float32, device=dev)
+
+    def _init_symmetric(self, dev):
+        import torch.distributed as dist
+        import torch.distributed._symmetric_memory as symm
+        group = self.group if self.group is not None else dist.group.WORLD
+        bufs, hdls = {}, {}
+        for name, numel in (("grad", self.P_pad), ("param", self.P_pad), ("flag", 32)):
+            t = symm.empty(numel, dtype=torch.float32, device=dev)
+            hdls[name] = symm.rendezvous(t, group)
+            bufs[name] = t
+        ptrs = {k: [int(x) for x in hdls[k].buffer_ptrs] for k in hdls}
+        if any(len(v) != self.world or not all(v) for v in ptrs.values()):
+            raise RuntimeError(f"symmetric memory rendezvous returned {ptrs}")
+        self.grad_flat, self.param_flat, self.flag_buf = bufs["grad"], bufs["param"], bufs["flag"]
+        self.grad_flat.zero_()
+        self.param_flat.zero_()
+        self.flag_buf.zero_()
+        self._peer_arrays = tuple((C.c_void_p * self.world)(*ptrs[k]) for k in ("grad", "param", "flag"))
+        self.p2p = hdls
+
+    def grads(self):
+        return [self.grad_flat]
+
+    def zero_grad(self, set_to_none=True):
+        for o in self.owners:
+            if not o.persistent:
+                o.param.grad = None
+
+    @torch.no_grad()
+    def step(self):
+        N.join_pending()
+        lib, st = N.lib(), N.stream()
+        for o, gview in zip(self.owners, self._grad_views):
+            if o.persistent:
+                continue
+            if o.param.grad is None:
+                raise RuntimeError("ShardedFlatAdam.step(): a parameter has no gradient (call backward first)")
+            gview.copy_(o.param.grad)
+        self.flag_buf[:1].zero_()
+        N.check(lib.lnrf_grad_nonfinite_check(C.cast(self._one_f32(self.grad_flat), C.c_void_p), 1, N.ptr(self.flag_buf), st))
+        if self.p2p is not None:
+            self.p2p["grad"].barrier(channel=0)   # every rank's gradient and flag are complete
+        g, p, f = self._peer_arrays
+        N.check(lib.lnrf_adam_step_sharded_f32(C.cast(g, C.c_void_p), C.cast(p, C.c_void_p), C.cast(f, C.c_void_p), self.world, self.rank,
+                                               self.lo, self.Sz, self._seg_start, self._seg_mult, len(self._seg_mult),
+                                               N.ptr(self.state[0]["exp_avg"]), N.ptr(self.state[0]["exp_avg_sq"]), self.lr, self.betas[0],
+                                               self.betas[1], self.eps, self.weight_decay, N.ptr(self._scale), N.ptr(self.found_inf),
+                                               N.ptr(self.step_count), N.ptr(self.lr_scale), st))
+        if self.p2p is not None:
+            self.p2p["grad"].barrier(channel=1)   # every rank has stored into this rank's parameters and read its gradient
+        # gradient clear (the fp32 vector as 2 x P_pad fp16 words) + GradScaler.update() in one launch
+        N.check(lib.lnrf_exchange_tail(N.ptr(self.grad_flat), 2 * self.P_pad, N.ptr(self._scale), N.ptr(self._growth_tracker),
+                                       N.ptr(self.found_inf), N.ptr(self.step_count), self.growth_factor, self.backoff_factor,
+                                       self.growth_interval, st))
+
+    def _one_f32(self, t):
+        arr = (N.OptTensor * 1)()
+        arr[0].grad, arr[0].n, arr[0].grad_dtype = t.data_ptr(), t.numel(), N.F32
+        return arr
+
+    # ---- checkpoints: torch.optim.Adam's per-parameter layout (a collective at world_size > 1) ------------------------
+    def _full(self, shard):
+        if self.world == 1:
+            return shard
+        import torch.distributed as dist
+        full = torch.empty(self.P_pad, dtype=shard.dtype, device=shard.device)
+        dist.all_gather_into_tensor(full, shard.contiguous(), group=self.group)
+        return full
+
+    def state_dict(self):
+        step = float(self.step_count.item()) - 1.0
+        ea, es = self._full(self.state[0]["exp_avg"]), self._full(self.state[0]["exp_avg_sq"])
+        state = {}
+        for i, (o, off) in enumerate(zip(self.owners, self._offsets)):
+            n = o.param.numel()
+            state[i] = {"step": torch.tensor(step), "exp_avg": ea[off:off + n].view_as(o.param).clone(),
+                        "exp_avg_sq": es[off:off + n].view_as(o.param).clone()}
+        groups = []
+        for gi in range(self.n_groups):
+            idx = [i for i, o in enumerate(self.owners) if o.group == gi]
+            mult = self.owners[idx[0]].lr_mult if idx else 1.0
+            groups.append({"lr": self.lr * mult, "betas": self.betas, "eps": self.eps, "weight_decay": self.weight_decay, "amsgrad": False,
+                           "maximize": False, "foreach": None, "capturable": False, "differentiable": False, "fused": None,
+                           "decoupled_weight_decay": False, "params": idx})
+        return {"state": state, "param_groups": groups}
+
+    @torch.no_grad()
+    def load_state_dict(self, sd):
+        n = len(self.owners)
+        if len(sd["state"]) not in (0, n):
+            raise RuntimeError(f"ShardedFlatAdam.load_state_dict: {len(sd['state'])} state entries for {n} parameter tensors")
+        if len(sd["state"]) == n:
+            for k in ("exp_avg", "exp_avg_sq"):
+                flat = torch.zeros(self.P_pad, dtype=torch.float32, device=self.param_flat.device)
+                for i, (o, off) in enumerate(zip(self.owners, self._offsets)):
+                    flat[off:off + o.param.numel()] = sd["state"][i][k].reshape(-1)
+                self.state[0][k].copy_(flat[self.lo:self.hi])
+            self.step_count.fill_(float(sd["state"][0]["step"]) + 1.0)
+        g = next((g for g in sd["param_groups"] if g["params"]), sd["param_groups"][0])
+        first = self.owners[g["params"][0]].lr_mult if g["params"] else 1.0
+        self.lr = float(g["lr"]) / first
+        self.betas, self.eps, self.weight_decay = tuple(map(float, g["betas"])), float(g["eps"]), float(g["weight_decay"])

@@ -158,19 +158,39 @@ class StyleTrainStep:
     palette -- inf check + unscale + Adam for all four tensors in 2 + 2 launches instead of torch's GradScaler + Adam passes
     (the reference's precision is kept: no autocast around the encoder, fp32 table and fp32 gradients, as nerf/utils.py:983 runs it).
     world_size > 1 = data parallel over VIEWS (SURVEY.md 8e): every rank trains on the masked points of its own view, gradients
-    are averaged across ranks inside optimizer.step()."""
+    are averaged across ranks inside optimizer.step().  With the fused optimizer that is `laenerf_b200.optim.ShardedFlatAdam`: the
+    parameters become views of one peer-mapped fp32 vector, the table gradient accumulates straight into a peer-mapped gradient
+    vector, and one kernel averages each rank's slice over NVLink, runs Adam on it and stores the result into every rank's
+    parameters.  Where torch symmetric memory is unavailable the gradients are all-reduced with NCCL instead, one collective per
+    tensor, and every rank runs the full Adam.  `exchange` records which path runs ("local", "p2p" or "allreduce"; for the last,
+    `p2p_error` says why)."""
 
     def __init__(self, style_encoder: LAENeRF, params=None, lr: float = 1e-3, fused_optimizer: bool = True, world_size: int = 1, rank: int = 0):
         self.model, self.params = style_encoder, params
         self.world = int(world_size)
         self.fused_optimizer = bool(fused_optimizer)
+        self.exchange, self.p2p_error = "local", None
         if self.fused_optimizer:
-            from .optim import AmpAdam
+            from .optim import AmpAdam, ShardedFlatAdam
             m = style_encoder
+            # get_params(): palette at 2 lr; the table's gradient reaches the sharded optimizer without autograd (persistent)
             owners = [(m.encoder, m.encoder.embeddings, 1.0, False, 0), (m.weight_net, m.weight_net.weights, 1.0, False, 1),
-                      (m.offset_net, m.offset_net.weights, 1.0, False, 2), (m, m.color_palette, 2.0, False, 3)]  # get_params(): palette at 2 lr
-            self.optimizer = AmpAdam(None, lr=lr, betas=(0.9, 0.999), eps=1e-8, fp16=True, world_size=1, rank=rank, owners=owners, n_groups=4)
-            self.optimizer.world = self.world  # fp32 tensors only: plain mean all-reduce of the gradients, replicated update
+                      (m.offset_net, m.offset_net.weights, 1.0, False, 2), (m, m.color_palette, 2.0, False, 3)]
+            self.optimizer = None
+            if self.world > 1:
+                try:
+                    self.optimizer = ShardedFlatAdam([(o[0], o[1], o[2], o[0] is m.encoder, o[4]) for o in owners], lr=lr, betas=(0.9, 0.999),
+                                                     eps=1e-8, world_size=self.world, rank=rank, n_groups=4)
+                    self.exchange = "p2p"
+                except Exception as e:  # never silently: the caller can report which exchange path ran
+                    self.p2p_error = f"{type(e).__name__}: {e}"[:300]
+            if self.optimizer is None:
+                self.optimizer = AmpAdam(None, lr=lr, betas=(0.9, 0.999), eps=1e-8, fp16=True, world_size=1, rank=rank, owners=owners,
+                                         n_groups=4)
+                self.optimizer.world = self.world  # fp32 tensors only: plain mean all-reduce of the gradients, replicated update
+                if self.world > 1:
+                    self.exchange = "allreduce"
+                    self.optimizer.p2p_error = self.p2p_error
             self.scaler = None
         else:
             self.optimizer = torch.optim.Adam(style_encoder.get_params(lr))
@@ -206,12 +226,15 @@ class GraphedStyleTrainStep:
     optimizer are ~60 launches of a few microseconds each, so issued from Python the iteration is bound by the interpreter (2.5 ms for
     49 152 points; the kernels take a fraction of that).  Inputs are copied into static device buffers; `loss` / `pred` are views of
     graph-owned memory that the next replay overwrites.  The point count is fixed per capture -- a view's masked points are padded or
-    chunked by the caller (the reference feeds one view's mask per step, nerf/utils.py:983-1034).  Single process only: the
-    data-parallel variant averages the fp32 gradients with an NCCL all-reduce per step and stays eager."""
+    chunked by the caller (the reference feeds one view's mask per step, nerf/utils.py:983-1034).  At world_size > 1 the step must
+    use the symmetric-memory exchange (`step.exchange == "p2p"`): the graph then holds the inf check, the two barriers around the
+    exchange kernel and the kernel itself, as GraphedTrainStep does for the NeRF; the NCCL fallback all-reduces eagerly and is
+    refused."""
 
     def __init__(self, step: StyleTrainStep, n_points: int):
-        if step.world > 1:
-            raise RuntimeError("GraphedStyleTrainStep: single-process only (the data-parallel step all-reduces its gradients eagerly)")
+        if step.world > 1 and step.exchange != "p2p":
+            raise RuntimeError("GraphedStyleTrainStep: at world_size > 1 the step must run the symmetric-memory exchange "
+                               f"(StyleTrainStep.exchange is {step.exchange!r}: {step.p2p_error})")
         self.step = step
         dev = next(step.model.parameters()).device
         self.x = torch.zeros(n_points, 3, device=dev)
