@@ -331,15 +331,17 @@ k_grid_bwd_tile(const typename Vec2<T>::type* __restrict__ grad, const float* __
             float2 acc[8];
             bool open = false;
             const bool slot_ok = PAIR && (reinterpret_cast<uintptr_t>(gg) & (2 * sizeof(T2) - 1)) == 0;
-            auto flush = [&]() {
+            // flush the corners c with (c & kmask) != kval: all of them for kmask = 0, kval = 1
+            auto flush = [&](uint32_t kmask, uint32_t kval) {
 #pragma unroll
                 for (int c = 0; c < 8; c += 2) {
+                    const bool f0 = ((uint32_t)c & kmask) != kval, f1 = ((uint32_t)(c + 1) & kmask) != kval;
                     const bool nz0 = acc[c].x != 0.f || acc[c].y != 0.f, nz1 = acc[c + 1].x != 0.f || acc[c + 1].y != 0.f;
-                    if (slot_ok && !(idx[c] & 1u) && idx[c + 1] == idx[c] + 1u) {
+                    if (f0 && f1 && slot_ok && !(idx[c] & 1u) && idx[c + 1] == idx[c] + 1u) {
                         if (nz0 || nz1) red4(gg + idx[c], acc[c], acc[c + 1]);
                     } else {
-                        if (nz0) red2(gg + idx[c], acc[c]);
-                        if (nz1) red2(gg + idx[c + 1], acc[c + 1]);
+                        if (f0 && nz0) red2(gg + idx[c], acc[c]);
+                        if (f1 && nz1) red2(gg + idx[c + 1], acc[c + 1]);
                     }
                 }
             };
@@ -356,12 +358,38 @@ k_grid_bwd_tile(const typename Vec2<T>::type* __restrict__ grad, const float* __
                 float pos[3];
                 cell_of<3, SMOOTH>(lv, x, align_corners, pg, pos, nullptr);
                 if (!open || pg[0] != cell[0] || pg[1] != cell[1] || pg[2] != cell[2]) {
-                    if (open) flush();
+                    // A neighbouring cell (every axis moved by at most one) shares a face, an edge or a vertex with the open one: those
+                    // corners are the same grid points, hence the same table entries, so their sums stay in registers instead of being
+                    // flushed.  Old corner c is kept iff (c & kmask) == kval, and becomes corner c ^ kmask of the new cell.
+                    uint32_t kmask = 0u, kval = 1u;  // nothing kept
+                    if (open) {
+                        uint32_t m = 0u, v = 0u;
+                        bool near = true;
+#pragma unroll
+                        for (int a = 0; a < 3; a++) {
+                            if (pg[a] == cell[a] + 1u) { m |= 1u << a; v |= 1u << a; }
+                            else if (pg[a] + 1u == cell[a]) m |= 1u << a;
+                            else if (pg[a] != cell[a]) near = false;
+                        }
+                        if (near) { kmask = m; kval = v; }
+                        flush(kmask, kval);
+                    }
+#pragma unroll
+                    for (int a = 0; a < 3; a++) {
+                        if (kmask & (1u << a)) {
+#pragma unroll
+                            for (int c = 0; c < 8; c++) {
+                                if (c & (1 << a)) continue;
+                                const float2 t = acc[c]; acc[c] = acc[c | (1 << a)]; acc[c | (1 << a)] = t;
+                            }
+                        }
+                    }
+#pragma unroll
+                    for (int c = 0; c < 8; c++)
+                        if (((uint32_t)c & kmask) != (kval ^ kmask)) acc[c] = make_float2(0.f, 0.f);
                     open = true;
                     cell[0] = pg[0]; cell[1] = pg[1]; cell[2] = pg[2];
                     corner_indices3(lv, pg, idx);
-#pragma unroll
-                    for (int c = 0; c < 8; c++) acc[c] = make_float2(0.f, 0.f);
                 }
 #pragma unroll
                 for (int c = 0; c < 8; c++) {
@@ -371,7 +399,7 @@ k_grid_bwd_tile(const typename Vec2<T>::type* __restrict__ grad, const float* __
                     acc[c].y = fmaf(w, gv.y, acc[c].y);
                 }
             }
-            if (open) flush();
+            if (open) flush(0u, 1u);
         }
     }
 }
