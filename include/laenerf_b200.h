@@ -310,6 +310,36 @@ LNRF_API int lnrf_grid_encode_backward_world(const void* grad, const float* inpu
                                              const int32_t* B_dev, uint32_t L, float S, uint32_t H, uint32_t gridtype,
                                              int align_corners, uint32_t interp, lnrf_dtype emb_dtype, lnrf_stream_t stream);
 
+/* Deterministic table gradient: what lnrf_grid_encode_backward / lnrf_grid_encode_backward_world compute, with a
+ * result that does not depend on the order of the reductions (the Python layer selects it when
+ * torch.are_deterministic_algorithms_enabled()).  Each flush adds round(p / q) to an int64 fixed-point sum with an
+ * integer reduction; lnrf_grid_det_finish then writes RN(grad_embeddings + sum * q), or NaN for an entry that received a
+ * non-finite contribution.  q = 2^(E + ceil(log2 B) + 1 - 62): E = 16 for fp16 gradients, for fp32 a pre-pass over the
+ * rows read writes the bit pattern of max finite |g| to *gmax (no host round trip).  DESIGN.md section 4.
+ *   acc   [entries * C] int64, 16-byte aligned; flags [entries] int32; gmax: one uint32 (fp32 gradients only, else NULL).
+ *   acc and flags must be zero on entry to the backward; the finish kernel zeroes every word it read, so they are
+ *   allocated zeroed once and stay armed.  B (capacity with B_dev) must be the same in the backward and the finish.
+ * grid_encode_backward_det: replaces lnrf_grid_encode_backward's table gradient (grad_embeddings is not an argument: it
+ * is written by the finish); dy_dx / grad_inputs as there. */
+LNRF_API int lnrf_grid_encode_backward_det(const void* grad, const float* inputs, const int32_t* offsets_host, void* acc,
+                                           void* flags, void* gmax, uint32_t B, uint32_t D, uint32_t C, uint32_t L, float S,
+                                           uint32_t H, const void* dy_dx, void* grad_inputs, uint32_t gridtype,
+                                           int align_corners, uint32_t interp, lnrf_dtype emb_dtype,
+                                           lnrf_grid_layout grad_layout, lnrf_stream_t stream);
+/* replaces lnrf_grid_encode_backward_world (rows at or past ceil128(*B_dev) are not read, by the pre-pass either) */
+LNRF_API int lnrf_grid_encode_backward_world_det(const void* grad, const float* inputs_world, float bound,
+                                                 const int32_t* offsets_host, void* acc, void* flags, void* gmax, uint32_t B,
+                                                 const int32_t* B_dev, uint32_t L, float S, uint32_t H, uint32_t gridtype,
+                                                 int align_corners, uint32_t interp, lnrf_dtype emb_dtype,
+                                                 lnrf_stream_t stream);
+/* grad_embeddings [entries, C] in emb_dtype: accumulated into (a zeroed buffer for a fresh gradient). */
+LNRF_API int lnrf_grid_det_finish(void* acc, void* flags, const void* gmax, uint32_t B, void* grad_embeddings,
+                                  uint32_t n_entries, uint32_t C, lnrf_dtype emb_dtype, lnrf_stream_t stream);
+/* 1 when lnrf_ffmlp_backward's weight gradient for this net is summed in a fixed order (the two-tile ReLU kernel),
+ * 0 when it takes the float-atomics kernel; < 0 for a shape lnrf_ffmlp_backward rejects. */
+LNRF_API int lnrf_ffmlp_backward_deterministic(uint32_t input_dim, uint32_t output_dim, uint32_t hidden_dim,
+                                               uint32_t num_layers, uint32_t activation, uint32_t output_activation);
+
 /* ---------------------------------------------------------------------------------------------------------
  * device-driven inference rounds (row f-3) -- the loop of NeRFRenderer.run_cuda / run_cuda_distill
  * (nerf/renderer.py:335-387, 425-470) without a device->host synchronisation per round.
@@ -444,6 +474,11 @@ LNRF_API int lnrf_occupancy_points(const int32_t* coords, const float* uniforms,
 /* tmp_grid_cascade[indices[i]] = sigmas[i] (renderer.py:601, 641). */
 LNRF_API int lnrf_occupancy_scatter(const float* sigmas, const int32_t* indices, uint32_t N, float* tmp_grid_cascade,
                                     lnrf_stream_t stream);
+/* Replaces lnrf_occupancy_scatter when results must not depend on timing: of duplicate indices the LAST occurrence wins, as
+ * torch's `tmp[idx] = sigma` does under torch.use_deterministic_algorithms(True).  winner: int32[cells] scratch, all -1
+ * on entry and re-armed to -1 on exit; indices outside [0, cells) are ignored. */
+LNRF_API int lnrf_occupancy_scatter_det(const float* sigmas, const int32_t* indices, uint32_t N, float* tmp_grid_cascade,
+                                        int32_t* winner, uint32_t cells, lnrf_stream_t stream);
 LNRF_API int lnrf_occupancy_fill(float* grid, uint32_t n, float value, lnrf_stream_t stream);
 /* density_grid = max(density_grid * decay, tmp_grid) where both >= 0 (renderer.py:625-626); tmp_grid is reset to -1;
  * mean_out[0] = mean(clamp(density_grid, 0)) (:627), mean_out[1] = min(mean, density_thresh) (:632), both on the device. */

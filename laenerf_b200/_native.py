@@ -100,6 +100,11 @@ SIGNATURES = {
     "lnrf_exchange_tail": (i32, [vp, u64, vp, vp, vp, vp, f32, f32, i32, vp]),
     "lnrf_amp_update": (i32, [vp, vp, vp, vp, f32, f32, i32, vp]),
     "lnrf_grad_nonfinite_check_amp_update": (i32, [vp, u32, vp, vp, vp, vp, f32, f32, i32, vp, vp]),
+    "lnrf_grid_encode_backward_det": (i32, [vp, vp, vp, vp, vp, vp, u32, u32, u32, u32, f32, u32, vp, vp, u32, i32, u32, i32, i32, vp]),
+    "lnrf_grid_encode_backward_world_det": (i32, [vp, vp, f32, vp, vp, vp, vp, u32, vp, u32, f32, u32, u32, i32, u32, i32, vp]),
+    "lnrf_grid_det_finish": (i32, [vp, vp, vp, u32, vp, u32, u32, i32, vp]),
+    "lnrf_ffmlp_backward_deterministic": (i32, [u32, u32, u32, u32, u32, u32]),
+    "lnrf_occupancy_scatter_det": (i32, [vp, vp, u32, vp, vp, u32, vp]),
 }
 
 class RenderDesc(C.Structure):
@@ -157,6 +162,22 @@ def lib():
 def check(status: int) -> None:
     if status != 0:
         raise RuntimeError(lib().lnrf_last_error().decode("utf-8", "replace"))
+
+
+def alert_not_deterministic(op: str) -> None:
+    """What torch does for its own ops without a deterministic kernel: under torch.use_deterministic_algorithms(True) raise a
+    RuntimeError naming the op, or warn when warn_only=True; nothing when the flag is off."""
+    import torch
+    if not torch.are_deterministic_algorithms_enabled():
+        return
+    msg = (f"{op} does not have a deterministic implementation, but you set 'torch.use_deterministic_algorithms(True)'. "
+           "You can turn off determinism just for this operation, or you can use the 'warn_only=True' option, if that's "
+           "acceptable for your application.")
+    if torch.is_deterministic_algorithms_warn_only_enabled():
+        import warnings
+        warnings.warn(msg, UserWarning, stacklevel=3)
+    else:
+        raise RuntimeError(msg)
 
 
 def ptr(t):

@@ -791,6 +791,14 @@ int mlp_shape(const char* who, uint32_t B, uint32_t input_dim, uint32_t output_d
     return check_mlp(who, B, input_dim, output_dim, 64, num_layers, 0, 6, sh);
 }
 
+// The two-tile ReLU kernel writes per-CTA slices that k_wgrad_reduce adds in a fixed order; every other net takes k_ffmlp_bwd, whose
+// weight gradient is a float atomicAdd per element (order-dependent).
+static bool bwd_fixed_order(const MlpShape& sh) {
+    const uint32_t nparams = 64u * (sh.in_dim + 64u * (sh.n_layers - 1) + sh.out_dim);
+    return sh.act == 0 && kBwdGroups * bwd2_group_cols(sh.in_dim, sh.out_dim, sh.n_layers) <= 512 && bwd2_smem_bytes(sh) <= 227 * 1024 &&
+           (kBwdGroups * (sh.n_layers + 2)) * kTileBytes >= 2 * nparams;
+}
+
 // One launch for the whole backward of a 64-wide net (+ the fp32 -> fp16 finalize of the weight gradients).  `glue` non-null
 // selects the colour-net variant with the NeRFNetwork glue fused in (see k_ffmlp_bwd).
 int ffmlp_bwd_run(const char* who, const void* grad_f16, const void* inputs_f16, const void* weights_f16, const void* forward_buffer_f16,
@@ -809,8 +817,7 @@ int ffmlp_bwd_run(const char* who, const void* grad_f16, const void* inputs_f16,
     const uint32_t nparams = (uint32_t)(need / sizeof(float) / kNumSMs);
     cudaError_t e = cudaSuccess;
     uint32_t nslices = 1;  // slices of partial sums the reduction adds up (the atomics path accumulates into one)
-    const bool relu2 = sh.act == 0 && kBwdGroups * bwd2_group_cols(input_dim, output_dim, num_layers) <= 512 &&
-                       bwd2_smem_bytes(sh) <= 227 * 1024 && (kBwdGroups * (num_layers + 2)) * kTileBytes >= 2 * nparams;
+    const bool relu2 = bwd_fixed_order(sh);
     LNRF_REQUIRE(!glue || relu2, "%s: the fused colour-net backward needs a ReLU net that fits the two-tile kernel", who);
     if (B > 0 && relu2) {
         const size_t smem = bwd2_smem_bytes(sh);
@@ -917,6 +924,14 @@ int lnrf_ffmlp_backward(const void* grad_f16, const void* inputs_f16, const void
     return lnrf::ffmlp_bwd_run("ffmlp_backward", grad_f16, inputs_f16, weights_f16, forward_buffer_f16, B, sh, calc_grad_inputs,
                                grad_inputs_f16, grad_weights_f16, wgrad_scratch, wgrad_scratch_bytes, nullptr, 0,
                                reinterpret_cast<cudaStream_t>(stream));
+}
+
+int lnrf_ffmlp_backward_deterministic(uint32_t input_dim, uint32_t output_dim, uint32_t hidden_dim, uint32_t num_layers, uint32_t activation,
+                                      uint32_t output_activation) {
+    MlpShape sh;
+    if (int e = check_mlp("ffmlp_backward_deterministic", 128, input_dim, output_dim, hidden_dim, num_layers, activation, output_activation, &sh))
+        return e;
+    return lnrf::bwd_fixed_order(sh) ? 1 : 0;
 }
 
 int lnrf_allocate_splitk(size_t size) { (void)size; return LNRF_OK; }

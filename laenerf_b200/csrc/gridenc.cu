@@ -14,6 +14,8 @@
 //   * everything else (D = 2, C in {1,4,8}, dy_dx, [L,B,C] layout) takes a generic thread-per-(sample, level) path.
 // Index arithmetic is uint32 and bit-identical to the reference (gridencoder.cu:50-84), including the per-level
 // scale evaluated on the device as fma(exp2f(level * S), H, -1).
+#include <cfloat>
+
 #include "common.cuh"
 
 namespace lnrf {
@@ -156,6 +158,41 @@ __device__ __forceinline__ void ld2x2(const float2* p, float2& a, float2& b) {
 __device__ __forceinline__ void red1(__half* p, float v) { atomicAdd(p, __float2half_rn(v)); }
 __device__ __forceinline__ void red1(float* p, float v) { atomicAdd(p, v); }
 
+// Deterministic table gradient (torch.use_deterministic_algorithms; DESIGN.md section 4, "Deterministic backward").  The fp32 value
+// a thread flushes depends only on the sample indices it owns (fixed 128-sample tile, fixed 8-sample run, fixed carry rule), never
+// on which CTA runs the tile; only the float reductions at L2 make the sum order-dependent.  Here a flush adds round(p / q) to an
+// int64 fixed-point sum instead, and integer addition is associative.  q = 2^qexp, qexp = E + ceil(log2 B) + 1 - 62 with 2^E >=
+// max |g| over the rows read: the corner weights of a sample sum to 1 within a level, so |sum| <= B * 2^E (1 + eps) < 2^62 q and
+// no int64 sum wraps.  A non-finite p sets its entry's flag instead (the finish kernel writes NaN there).
+struct DetSink {
+    unsigned long long* acc;  // [entries, C] two's-complement fixed-point sums, zero between calls (k_det_finish re-arms them)
+    uint32_t* flag;           // [entries] non-zero: a contribution was non-finite; zero between calls
+    const uint32_t* gmax;     // fp32 gradients: bit pattern of max finite |g| (k_det_absmax); nullptr: fp16, |g| < 2^16
+    int lb;                   // ceil(log2 B), B = the row capacity of the call
+};
+constexpr int kDetMinExp = -60;  // E for an all-zero gradient: keeps 2^-qexp a normal float
+
+__device__ __forceinline__ int det_qexp(const DetSink& d) {
+    int E = 16;
+    if (d.gmax) {
+        const uint32_t m = *d.gmax;  // 2^((m >> 23) - 126) > m for every finite non-negative float
+        E = m == 0u ? kDetMinExp : max((int)(m >> 23) - 126, kDetMinExp);
+    }
+    return E + d.lb + 1 - 62;
+}
+__device__ __forceinline__ float det_inv_q(const DetSink& d) { return __int_as_float((127 - det_qexp(d)) << 23); }  // exact 2^-qexp
+
+__device__ __forceinline__ void det_red(unsigned long long* p, float v, float inv_q) {
+    const long long q = __float2ll_rn(__fmul_rn(v, inv_q));  // the multiply by a power of two is exact
+    if (q) asm volatile("red.global.add.u64 [%0], %1;" ::"l"(p), "l"(q) : "memory");
+}
+// entry e of a C = 2 table
+__device__ __forceinline__ void det_add2(const DetSink& d, size_t e, float2 v, float inv_q) {
+    if (!isfinite(v.x) || !isfinite(v.y)) { d.flag[e] = 1u; return; }
+    det_red(d.acc + e * 2, v.x, inv_q);
+    det_red(d.acc + e * 2 + 1, v.y, inv_q);
+}
+
 // position inside the level: cell + interpolation weights (gridencoder.cu:141-163)
 template <int D, bool SMOOTH>
 __device__ __forceinline__ void cell_of(const Level& lv, const float* x, bool align_corners, uint32_t* pg, float* pos,
@@ -283,12 +320,13 @@ k_grid_fwd_tile(const float* __restrict__ inputs, const typename Vec2<T>::type* 
 // levels (level 0 has 4920 entries for 2.3e5 samples x 8 corners) -- the reference issues every one of them.
 constexpr int kRun = 8;
 
-template <typename T, bool SMOOTH, bool PAIR>
+// DET: the flushes go to the fixed-point sums of `det` (see DetSink) instead of reductions into grad_emb.
+template <typename T, bool SMOOTH, bool PAIR, bool DET>
 __global__ void __launch_bounds__(kGridThreads)
 k_grid_bwd_tile(const typename Vec2<T>::type* __restrict__ grad, const float* __restrict__ inputs,
                 typename Vec2<T>::type* __restrict__ grad_emb, const uint32_t B, const uint32_t L, const float S,
                 const uint32_t H, const uint32_t gridtype, const bool align_corners, const GridOffsets off,
-                uint32_t ntiles, const float in_bound, const int* __restrict__ B_dev) {
+                uint32_t ntiles, const float in_bound, const int* __restrict__ B_dev, const DetSink det) {
     using T2 = typename Vec2<T>::type;
     extern __shared__ __align__(16) unsigned char s_raw[];
     __shared__ Level s_lv[kMaxLevels];
@@ -306,6 +344,8 @@ k_grid_bwd_tile(const typename Vec2<T>::type* __restrict__ grad, const float* __
     const uint32_t LP = L | 1u;
     const int tid = threadIdx.x;
     if (tid < (int)L) s_lv[tid] = make_level<3>(tid, S, H, off, gridtype, align_corners);
+    float inv_q = 0.0f;
+    if constexpr (DET) inv_q = det_inv_q(det);  // after pdl_wait: the max pre-pass ran ahead on the stream
 
     for (uint32_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         const size_t b0 = (size_t)tile * kTile;
@@ -337,7 +377,10 @@ k_grid_bwd_tile(const typename Vec2<T>::type* __restrict__ grad, const float* __
                 for (int c = 0; c < 8; c += 2) {
                     const bool f0 = ((uint32_t)c & kmask) != kval, f1 = ((uint32_t)(c + 1) & kmask) != kval;
                     const bool nz0 = acc[c].x != 0.f || acc[c].y != 0.f, nz1 = acc[c + 1].x != 0.f || acc[c + 1].y != 0.f;
-                    if (f0 && f1 && slot_ok && !(idx[c] & 1u) && idx[c + 1] == idx[c] + 1u) {
+                    if constexpr (DET) {  // no 64-bit vector reduction exists: one per corner and channel
+                        if (f0 && nz0) det_add2(det, (size_t)lv.base + idx[c], acc[c], inv_q);
+                        if (f1 && nz1) det_add2(det, (size_t)lv.base + idx[c + 1], acc[c + 1], inv_q);
+                    } else if (f0 && f1 && slot_ok && !(idx[c] & 1u) && idx[c + 1] == idx[c] + 1u) {
                         if (nz0 || nz1) red4(gg + idx[c], acc[c], acc[c + 1]);
                     } else {
                         if (f0 && nz0) red2(gg + idx[c], acc[c]);
@@ -484,11 +527,11 @@ k_grid_fwd_generic(const float* __restrict__ inputs, const T* __restrict__ emb, 
     }
 }
 
-template <typename T, int D, int C, bool SMOOTH>
+template <typename T, int D, int C, bool SMOOTH, bool DET>
 __global__ void __launch_bounds__(256)
 k_grid_bwd_generic(const T* __restrict__ grad, const float* __restrict__ inputs, T* __restrict__ grad_emb, const uint32_t B,
                    const uint32_t L, const float S, const uint32_t H, const uint32_t gridtype, const bool align_corners,
-                   const GridOffsets off, const int layout) {
+                   const GridOffsets off, const int layout, const DetSink det) {
     const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
     const uint32_t level = blockIdx.y;
     if (b >= B) return;
@@ -516,8 +559,18 @@ k_grid_bwd_generic(const T* __restrict__ grad, const float* __restrict__ inputs,
             if (c & (1 << d)) { w *= pos[d]; pgl[d] = pg[d] + 1; }
             else { w *= 1.0f - pos[d]; pgl[d] = pg[d]; }
         }
-        const size_t index = (size_t)grid_index<D>(lv, pgl) * C;
-        if (C % 2 == 0) {
+        const uint32_t entry = grid_index<D>(lv, pgl);
+        const size_t index = (size_t)entry * C;
+        if constexpr (DET) {
+            const size_t e = (size_t)lv.base + entry;
+            const float inv_q = det_inv_q(det);
+#pragma unroll
+            for (int ch = 0; ch < C; ch++) {
+                const float v = w * gv[ch];
+                if (!isfinite(v)) det.flag[e] = 1u;
+                else det_red(det.acc + e * C + ch, v, inv_q);
+            }
+        } else if (C % 2 == 0) {
             using T2 = typename Vec2<T>::type;
 #pragma unroll
             for (int ch = 0; ch < C; ch += 2) red2(reinterpret_cast<T2*>(gg + index + ch), make_float2(w * gv[ch], w * gv[ch + 1]));
@@ -598,6 +651,46 @@ k_grid_grad_tv(const T* __restrict__ inputs, const T* __restrict__ emb, T* __res
     for (int ch = 0; ch < C; ch++) red1(gg + index + ch, w * results[ch] * rsqrtf(idelta[ch] + 1e-9f));
 }
 
+// max finite |g| over the first n elements (n cut to the live 128-row tiles when B_dev is given), as float bits: non-negative floats
+// order like their bit patterns, so one integer max per warp; *gmax must be zero on entry.  Order-independent.
+__global__ void __launch_bounds__(256)
+k_det_absmax(const float* __restrict__ g, size_t n, const uint32_t row_elems, const int* __restrict__ B_dev, uint32_t* __restrict__ gmax) {
+    if (B_dev) {
+        const size_t live = (size_t)div_up((uint32_t)max(*B_dev, 0), (uint32_t)kTile) * kTile * row_elems;
+        n = live < n ? live : n;
+    }
+    float m = 0.0f;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        const float v = fabsf(__ldcs(g + i));
+        if (v <= FLT_MAX) m = fmaxf(m, v);  // non-finite values set flags, they do not scale the quantum
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(kFull, m, o));
+    if ((threadIdx.x & 31) == 0 && m > 0.0f) atomicMax(gmax, __float_as_uint(m));
+}
+
+__device__ __forceinline__ void from_d(double v, __half& o) { o = __double2half(v); }
+__device__ __forceinline__ void from_d(double v, float& o) { o = __double2float_rn(v); }
+
+// out[e, ch] = RN_T(out[e, ch] + acc[e, ch] * q), or NaN for a flagged entry; the acc / flag words read are zeroed for the next call.
+// Entries with nothing to add are left untouched (out + 0 is out).
+template <typename T>
+__global__ void __launch_bounds__(256)
+k_det_finish(const DetSink d, T* __restrict__ out, const uint32_t n_entries, const uint32_t C) {
+    const int qexp = det_qexp(d);
+    for (uint32_t e = blockIdx.x * blockDim.x + threadIdx.x; e < n_entries; e += gridDim.x * blockDim.x) {
+        const bool bad = d.flag[e] != 0u;
+        if (bad) d.flag[e] = 0u;
+        for (uint32_t ch = 0; ch < C; ch++) {
+            const size_t i = (size_t)e * C + ch;
+            const long long a = (long long)d.acc[i];
+            if (a) d.acc[i] = 0ull;
+            if (bad) from_f(__int_as_float(0x7fffffff), out[i]);
+            else if (a) from_d((double)to_f(out[i]) + ldexp((double)a, qexp), out[i]);
+        }
+    }
+}
+
 __global__ void k_grid_level_scales(uint32_t L, float S, uint32_t H, float* __restrict__ scales) {
     const uint32_t l = threadIdx.x;
     if (l < L) scales[l] = __fmaf_rn(exp2f(__fmul_rn((float)l, S)), (float)H, -1.0f);
@@ -647,9 +740,15 @@ static void launch_fwd_generic(bool smooth, dim3 g, cudaStream_t st, const float
 }
 template <typename T, int D, int C>
 static void launch_bwd_generic(bool smooth, dim3 g, cudaStream_t st, const T* grad, const float* in, T* ge, uint32_t B, uint32_t L,
-                               float S, uint32_t H, uint32_t gridtype, bool ac, const GridOffsets& off, int layout) {
-    if (smooth) k_grid_bwd_generic<T, D, C, true><<<g, 256, 0, st>>>(grad, in, ge, B, L, S, H, gridtype, ac, off, layout);
-    else k_grid_bwd_generic<T, D, C, false><<<g, 256, 0, st>>>(grad, in, ge, B, L, S, H, gridtype, ac, off, layout);
+                               float S, uint32_t H, uint32_t gridtype, bool ac, const GridOffsets& off, int layout, const DetSink* det) {
+    const DetSink d = det ? *det : DetSink{};
+    if (det) {
+        if (smooth) k_grid_bwd_generic<T, D, C, true, true><<<g, 256, 0, st>>>(grad, in, ge, B, L, S, H, gridtype, ac, off, layout, d);
+        else k_grid_bwd_generic<T, D, C, false, true><<<g, 256, 0, st>>>(grad, in, ge, B, L, S, H, gridtype, ac, off, layout, d);
+    } else {
+        if (smooth) k_grid_bwd_generic<T, D, C, true, false><<<g, 256, 0, st>>>(grad, in, ge, B, L, S, H, gridtype, ac, off, layout, d);
+        else k_grid_bwd_generic<T, D, C, false, false><<<g, 256, 0, st>>>(grad, in, ge, B, L, S, H, gridtype, ac, off, layout, d);
+    }
 }
 
 #define LNRF_DISPATCH_DC(D, C, CALL)                                                       \
@@ -691,29 +790,40 @@ static int grid_forward_t(const float* inputs, const T* emb, const GridOffsets& 
     return LNRF_OK;
 }
 
+// det != nullptr: the table gradient goes to det's fixed-point sums (grad_emb is not touched; k_det_finish writes it)
 template <typename T>
 static int grid_backward_t(const T* grad, const float* inputs, const GridOffsets& off, T* grad_emb, uint32_t B, uint32_t D, uint32_t C,
                            uint32_t L, float S, uint32_t H, const T* dy_dx, T* grad_inputs, uint32_t gridtype, bool ac, uint32_t interp,
-                           int layout, cudaStream_t st, float in_bound = 0.0f, const int* B_dev = nullptr) {
+                           int layout, cudaStream_t st, float in_bound = 0.0f, const int* B_dev = nullptr, const DetSink* det = nullptr) {
     using T2 = typename Vec2<T>::type;
     const bool smooth = interp == 1;
-    const bool hot = D == 3 && C == 2 && layout == LNRF_GRID_BLC && (reinterpret_cast<uintptr_t>(grad_emb) % sizeof(T2)) == 0 &&
+    const bool hot = D == 3 && C == 2 && layout == LNRF_GRID_BLC && (det || (reinterpret_cast<uintptr_t>(grad_emb) % sizeof(T2)) == 0) &&
                      (reinterpret_cast<uintptr_t>(grad) % sizeof(T2)) == 0;
     if ((in_bound > 0.0f || B_dev) && (!hot || dy_dx)) {
         set_error("grid_encode_backward: in_bound / device-side B need the D=3, C=2, [B, L*C] kernel without input gradients");
         return LNRF_ERR_UNSUPPORTED;
     }
+    if (det && det->gmax) {  // fp32 gradients: the quantum follows max |g| over the rows the backward reads (no host round trip)
+        cudaError_t e = cudaMemsetAsync(const_cast<uint32_t*>(det->gmax), 0, sizeof(uint32_t), st);
+        if (e != cudaSuccess) return cuda_fail(e, "grid_encode_backward(det)");
+        const size_t n = (size_t)B * L * C;
+        const size_t want = (n + 255) / 256, cap = (size_t)kNumSMs * 4;
+        k_det_absmax<<<(uint32_t)(want < cap ? want : cap), 256, 0, st>>>(reinterpret_cast<const float*>(grad), n, L * C, B_dev,
+                                                                         const_cast<uint32_t*>(det->gmax));
+        LNRF_LAUNCH_CHECK("grid_encode_backward(max |g|)");
+    }
     if (hot) {
         const uint32_t ntiles = div_up(B, (uint32_t)kTile);
         const uint32_t grid = tile_grid(ntiles, 1);
         const size_t smem = (size_t)kTile * (L | 1u) * sizeof(T2);
-        auto kern = smooth ? (pair_mode() & 2 ? k_grid_bwd_tile<T, true, true> : k_grid_bwd_tile<T, true, false>)
-                           : (pair_mode() & 2 ? k_grid_bwd_tile<T, false, true> : k_grid_bwd_tile<T, false, false>);
+        auto kern = det ? (smooth ? k_grid_bwd_tile<T, true, false, true> : k_grid_bwd_tile<T, false, false, true>)
+                  : smooth ? (pair_mode() & 2 ? k_grid_bwd_tile<T, true, true, false> : k_grid_bwd_tile<T, true, false, false>)
+                           : (pair_mode() & 2 ? k_grid_bwd_tile<T, false, true, false> : k_grid_bwd_tile<T, false, false, false>);
         launch_pdl(kern, grid, kGridThreads, smem, st, reinterpret_cast<const T2*>(grad), inputs, reinterpret_cast<T2*>(grad_emb), B, L, S, H, gridtype,
-                                               ac, off, ntiles, in_bound, B_dev);
+                                               ac, off, ntiles, in_bound, B_dev, det ? *det : DetSink{});
     } else {
         const dim3 g(div_up(B, 256u), L, 1);
-#define CALL_(DD, CC) launch_bwd_generic<T, DD, CC>(smooth, g, st, grad, inputs, grad_emb, B, L, S, H, gridtype, ac, off, layout)
+#define CALL_(DD, CC) launch_bwd_generic<T, DD, CC>(smooth, g, st, grad, inputs, grad_emb, B, L, S, H, gridtype, ac, off, layout, det)
         LNRF_DISPATCH_DC(D, C, CALL_);
 #undef CALL_
     }
@@ -808,6 +918,68 @@ int lnrf_grid_encode_backward(const void* grad, const float* inputs, const void*
                                       (float*)grad_inputs, gridtype, align_corners != 0, interp, (int)grad_layout, S_(stream));
     set_error("grid_encode_backward: unsupported embedding dtype %d", (int)emb_dtype);
     return LNRF_ERR_UNSUPPORTED;
+}
+
+// ---- deterministic table gradient (DetSink) ----
+static int det_sink(const char* who, void* acc, void* flags, void* gmax, uint32_t B, lnrf_dtype dt, DetSink* d) {
+    LNRF_REQUIRE(acc && flags, "%s: acc / flags is null", who);
+    LNRF_REQUIRE(dt == LNRF_F16 || dt == LNRF_F32, "%s: unsupported dtype %d", who, (int)dt);
+    LNRF_REQUIRE(dt == LNRF_F16 || gmax, "%s: fp32 gradients need the gmax word", who);
+    LNRF_REQUIRE((reinterpret_cast<uintptr_t>(acc) & 15) == 0, "%s: acc must be 16-byte aligned", who);
+    LNRF_REQUIRE(B >= 1, "%s: B must be >= 1", who);
+    int lb = 0;
+    while ((1ull << lb) < (unsigned long long)B) lb++;
+    *d = DetSink{(unsigned long long*)acc, (uint32_t*)flags, dt == LNRF_F32 ? (const uint32_t*)gmax : nullptr, lb};
+    return LNRF_OK;
+}
+
+int lnrf_grid_encode_backward_det(const void* grad, const float* inputs, const int32_t* offsets_host, void* acc, void* flags, void* gmax,
+                                  uint32_t B, uint32_t D, uint32_t C, uint32_t L, float S, uint32_t H, const void* dy_dx, void* grad_inputs,
+                                  uint32_t gridtype, int align_corners, uint32_t interp, lnrf_dtype emb_dtype, lnrf_grid_layout grad_layout,
+                                  lnrf_stream_t stream) {
+    GridOffsets off;
+    if (int e = check_grid_args("grid_encode_backward_det", offsets_host, D, C, L, gridtype, interp, &off)) return e;
+    if (B == 0) return LNRF_OK;
+    LNRF_REQUIRE(grad && inputs, "grid_encode_backward_det: null pointer");
+    LNRF_REQUIRE((uint64_t)B * L * C < (1ull << 40), "grid_encode_backward_det: batch too large");
+    DetSink d;
+    if (int e = det_sink("grid_encode_backward_det", acc, flags, gmax, B, emb_dtype, &d)) return e;
+    if (emb_dtype == LNRF_F16)
+        return grid_backward_t<__half>((const __half*)grad, inputs, off, nullptr, B, D, C, L, S, H, (const __half*)dy_dx, (__half*)grad_inputs,
+                                       gridtype, align_corners != 0, interp, (int)grad_layout, S_(stream), 0.0f, nullptr, &d);
+    return grid_backward_t<float>((const float*)grad, inputs, off, nullptr, B, D, C, L, S, H, (const float*)dy_dx, (float*)grad_inputs,
+                                  gridtype, align_corners != 0, interp, (int)grad_layout, S_(stream), 0.0f, nullptr, &d);
+}
+
+int lnrf_grid_encode_backward_world_det(const void* grad, const float* inputs_world, float bound, const int32_t* offsets_host, void* acc,
+                                        void* flags, void* gmax, uint32_t B, const int32_t* B_dev, uint32_t L, float S, uint32_t H,
+                                        uint32_t gridtype, int align_corners, uint32_t interp, lnrf_dtype emb_dtype, lnrf_stream_t stream) {
+    GridOffsets off;
+    if (int e = check_grid_args("grid_encode_backward_world_det", offsets_host, 3, 2, L, gridtype, interp, &off)) return e;
+    if (B == 0) return LNRF_OK;
+    LNRF_REQUIRE(grad && inputs_world && bound > 0.0f, "grid_encode_backward_world_det: null pointer / bound <= 0");
+    DetSink d;
+    if (int e = det_sink("grid_encode_backward_world_det", acc, flags, gmax, B, emb_dtype, &d)) return e;
+    if (emb_dtype == LNRF_F16)
+        return grid_backward_t<__half>((const __half*)grad, inputs_world, off, nullptr, B, 3, 2, L, S, H, nullptr, nullptr, gridtype,
+                                       align_corners != 0, interp, (int)LNRF_GRID_BLC, S_(stream), bound, B_dev, &d);
+    return grid_backward_t<float>((const float*)grad, inputs_world, off, nullptr, B, 3, 2, L, S, H, nullptr, nullptr, gridtype,
+                                  align_corners != 0, interp, (int)LNRF_GRID_BLC, S_(stream), bound, B_dev, &d);
+}
+
+int lnrf_grid_det_finish(void* acc, void* flags, const void* gmax, uint32_t B, void* grad_embeddings, uint32_t n_entries, uint32_t C,
+                         lnrf_dtype emb_dtype, lnrf_stream_t stream) {
+    LNRF_REQUIRE(C == 1 || C == 2 || C == 4 || C == 8, "grid_det_finish: C must be 1, 2, 4, or 8");
+    LNRF_REQUIRE(grad_embeddings || n_entries == 0, "grid_det_finish: grad_embeddings is null");
+    DetSink d;
+    if (int e = det_sink("grid_det_finish", acc, flags, const_cast<void*>(gmax), B, emb_dtype, &d)) return e;
+    if (n_entries == 0) return LNRF_OK;
+    const uint32_t want = div_up(n_entries, 256u), cap = (uint32_t)kNumSMs * 16u;
+    const uint32_t g = want < cap ? want : cap;
+    if (emb_dtype == LNRF_F16) k_det_finish<__half><<<g, 256, 0, S_(stream)>>>(d, (__half*)grad_embeddings, n_entries, C);
+    else k_det_finish<float><<<g, 256, 0, S_(stream)>>>(d, (float*)grad_embeddings, n_entries, C);
+    LNRF_LAUNCH_CHECK("grid_det_finish");
+    return LNRF_OK;
 }
 
 int lnrf_grad_total_variation(const void* inputs, const void* embeddings, void* grad, const int32_t* offsets_host, float weight,

@@ -47,6 +47,25 @@ k_occ_scatter(const float* __restrict__ sigmas, const int* __restrict__ indices,
     if (i < N) tmp_cas[indices[i]] = sigmas[i];
 }
 
+// Duplicate indices resolved as torch's deterministic `tmp[idx] = sigma` does (the last occurrence wins): the largest sample index per
+// cell is found with an integer max, then only that sample stores.  `winner` (int32 per cell) is -1 on entry and re-armed on exit.
+__global__ void __launch_bounds__(256)
+k_occ_scatter_claim(const int* __restrict__ indices, const uint32_t N, const uint32_t cells, int* __restrict__ winner) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < N && (uint32_t)indices[i] < cells) atomicMax(winner + indices[i], (int)i);
+}
+__global__ void __launch_bounds__(256)
+k_occ_scatter_store(const float* __restrict__ sigmas, const int* __restrict__ indices, const uint32_t N, const uint32_t cells,
+                    int* __restrict__ winner, float* __restrict__ tmp_cas) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N) return;
+    const int idx = indices[i];
+    if ((uint32_t)idx < cells && winner[idx] == (int)i) {  // a loser never reads its own index back, re-armed or not
+        tmp_cas[idx] = sigmas[i];
+        winner[idx] = -1;
+    }
+}
+
 __global__ void __launch_bounds__(256) k_occ_fill(float* __restrict__ p, const uint32_t n, const float v) {
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) p[i] = v;
 }
@@ -197,6 +216,18 @@ int lnrf_occupancy_scatter(const float* sigmas, const int32_t* indices, uint32_t
     LNRF_REQUIRE(sigmas && indices && tmp_grid_cascade, "occupancy_scatter: null pointer");
     k_occ_scatter<<<div_up(N, 256u), 256, 0, S(stream)>>>(sigmas, indices, N, tmp_grid_cascade);
     LNRF_LAUNCH_CHECK("occupancy_scatter");
+    return LNRF_OK;
+}
+
+int lnrf_occupancy_scatter_det(const float* sigmas, const int32_t* indices, uint32_t N, float* tmp_grid_cascade, int32_t* winner,
+                               uint32_t cells, lnrf_stream_t stream) {
+    if (N == 0) return LNRF_OK;
+    LNRF_REQUIRE(sigmas && indices && tmp_grid_cascade && winner, "occupancy_scatter_det: null pointer");
+    LNRF_REQUIRE(cells > 0 && N <= 0x7fffffffu, "occupancy_scatter_det: cells must be > 0 and N < 2^31");
+    k_occ_scatter_claim<<<div_up(N, 256u), 256, 0, S(stream)>>>(indices, N, cells, winner);
+    LNRF_LAUNCH_CHECK("occupancy_scatter_det(claim)");
+    k_occ_scatter_store<<<div_up(N, 256u), 256, 0, S(stream)>>>(sigmas, indices, N, cells, winner, tmp_grid_cascade);
+    LNRF_LAUNCH_CHECK("occupancy_scatter_det");
     return LNRF_OK;
 }
 

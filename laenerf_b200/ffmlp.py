@@ -44,9 +44,13 @@ class _ffmlp_forward(Function):
         grad = grad.contiguous().half()
         inputs, weights, outputs, forward_buffer = ctx.saved_tensors
         input_dim, output_dim, hidden_dim, num_layers, activation, output_activation, calc_grad_inputs = ctx.dims
+        lib = N.lib()
+        if torch.are_deterministic_algorithms_enabled() and not backward_deterministic(input_dim, output_dim, hidden_dim, num_layers,
+                                                                                      activation, output_activation):
+            N.alert_not_deterministic(f"FFMLP backward of a {input_dim}-{hidden_dim}x{num_layers}-{output_dim} net with activation "
+                                      f"{activation} (lnrf_ffmlp_backward, float-atomics weight gradient)")
         grad_inputs = torch.empty_like(inputs) if calc_grad_inputs else None
         grad_weights = torch.empty_like(weights)
-        lib = N.lib()
         nbytes = lib.lnrf_ffmlp_wgrad_scratch_bytes(input_dim, output_dim, hidden_dim, num_layers)
         scratch = torch.empty(nbytes // 4, dtype=torch.float32, device=grad.device)
         N.check(lib.lnrf_ffmlp_backward(N.ptr(grad), N.ptr(inputs), N.ptr(weights), N.ptr(forward_buffer), B, input_dim,
@@ -57,6 +61,14 @@ class _ffmlp_forward(Function):
 
 
 ffmlp_forward = _ffmlp_forward.apply
+
+
+def backward_deterministic(input_dim, output_dim, hidden_dim, num_layers, activation, output_activation=6) -> bool:
+    """Whether lnrf_ffmlp_backward sums this net's weight gradient in a fixed order (the two-tile ReLU kernel) rather than with
+    float atomics."""
+    r = N.lib().lnrf_ffmlp_backward_deterministic(input_dim, output_dim, hidden_dim, num_layers, activation, output_activation)
+    N.check(min(r, 0))
+    return r == 1
 
 
 def convert_activation(act):  # ffmlp.py:89-96

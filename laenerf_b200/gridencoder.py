@@ -41,6 +41,22 @@ def _offsets_host(offsets: torch.Tensor) -> torch.Tensor:
     return h
 
 
+class DeterministicWorkspace:
+    """State of the deterministic table gradient (include/laenerf_b200.h, lnrf_grid_encode_backward_det): int64 fixed-point
+    sums [entries, C], a non-finite flag per entry and the max-|g| word of fp32 gradients.  Allocated zeroed once; the finish
+    kernel re-arms every word it reads, so a step needs no memset and the buffers can live inside a captured graph."""
+
+    def __init__(self):
+        self.acc = self.flags = self.gmax = None
+
+    def get(self, entries: int, C: int, dev):
+        if self.acc is None or self.acc.shape != (entries, C) or self.acc.device != dev:
+            self.acc = torch.zeros(entries, C, dtype=torch.int64, device=dev)
+            self.flags = torch.zeros(entries, dtype=torch.int32, device=dev)
+            self.gmax = torch.zeros(1, dtype=torch.int32, device=dev)
+        return self.acc, self.flags, self.gmax
+
+
 def _dt(t: torch.Tensor) -> int:
     if t.dtype == torch.float16:
         return N.F16
@@ -53,7 +69,8 @@ class _grid_encode(Function):
     @staticmethod
     @custom_fwd(device_type="cuda")
     def forward(ctx, inputs, embeddings, offsets, per_level_scale, base_resolution, calc_grad_inputs=False, gridtype=0,
-                align_corners=False, interpolation=0, shadow_f16=None, grad_f16=None, world_bound=0.0, b_dev=None, grad_f32=None):
+                align_corners=False, interpolation=0, shadow_f16=None, grad_f16=None, world_bound=0.0, b_dev=None, grad_f32=None,
+                det_ws=None):
         # b_dev: optional device int32 with the number of live rows (world_bound > 0 only): whole 128-row tiles past it are neither
         # encoded nor differentiated -- their output rows stay unwritten, which is fine for a consumer that honours the same count
         # world_bound > 0: `inputs` are world coordinates and the kernel applies GridEncoder.forward's (x + bound) / (2 * bound)
@@ -91,6 +108,7 @@ class _grid_encode(Function):
         ctx.dims = [B, D, C, L, S, H, gridtype, interpolation]
         ctx.world_bound = float(world_bound)
         ctx.align_corners = align_corners
+        ctx.det_ws = det_ws  # GridEncoder's DeterministicWorkspace (None: a fresh one per deterministic backward)
         return outputs
 
     @staticmethod
@@ -105,7 +123,24 @@ class _grid_encode(Function):
         # ShardedFlatAdam into this rank's fp32 gradient vector, which the other ranks read over NVLink
         grad_embeddings = ctx.grad_buf if ctx.grad_buf is not None else torch.zeros_like(embeddings)
         grad_inputs = torch.zeros_like(inputs, dtype=embeddings.dtype) if dy_dx is not None else None
-        if ctx.world_bound > 0:
+        if torch.are_deterministic_algorithms_enabled():
+            # fixed-point integer sums: the table gradient does not depend on the order of the reductions (DESIGN.md section 4)
+            ws = ctx.det_ws if ctx.det_ws is not None else DeterministicWorkspace()
+            acc, flags, gmax = ws.get(embeddings.shape[0], C, embeddings.device)
+            gm = gmax if embeddings.dtype == torch.float32 else None
+            if ctx.world_bound > 0:
+                N.check(N.lib().lnrf_grid_encode_backward_world_det(N.ptr(grad), N.ptr(inputs), ctx.world_bound, N.ptr(_offsets_host(offsets)),
+                                                                    N.ptr(acc), N.ptr(flags), N.ptr(gm), B, N.ptr(b_dev), L, S, H, int(gridtype),
+                                                                    int(bool(ctx.align_corners)), int(interpolation), _dt(embeddings), N.stream()))
+            else:
+                N.check(N.lib().lnrf_grid_encode_backward_det(N.ptr(grad), N.ptr(inputs), N.ptr(_offsets_host(offsets)), N.ptr(acc), N.ptr(flags),
+                                                              N.ptr(gm), B, D, C, L, S, H, N.ptr(dy_dx), N.ptr(grad_inputs), int(gridtype),
+                                                              int(bool(ctx.align_corners)), int(interpolation), _dt(embeddings), N.GRID_BLC,
+                                                              N.stream()))
+            if B > 0:
+                N.check(N.lib().lnrf_grid_det_finish(N.ptr(acc), N.ptr(flags), N.ptr(gm), B, N.ptr(grad_embeddings), embeddings.shape[0], C,
+                                                     _dt(embeddings), N.stream()))
+        elif ctx.world_bound > 0:
             N.check(N.lib().lnrf_grid_encode_backward_world(N.ptr(grad), N.ptr(inputs), ctx.world_bound, N.ptr(_offsets_host(offsets)),
                                                             N.ptr(grad_embeddings), B, N.ptr(b_dev), L, S, H, int(gridtype),
                                                             int(bool(ctx.align_corners)), int(interpolation), _dt(embeddings), N.stream()))
@@ -118,7 +153,7 @@ class _grid_encode(Function):
             grad_inputs = grad_inputs.to(inputs.dtype)
         if ctx.grad_buf is not None:
             grad_embeddings = None
-        return grad_inputs, grad_embeddings, None, None, None, None, None, None, None, None, None, None, None, None
+        return grad_inputs, grad_embeddings, None, None, None, None, None, None, None, None, None, None, None, None, None
 
 
 grid_encode = _grid_encode.apply
@@ -162,6 +197,7 @@ class GridEncoder(nn.Module):
         self._grad_f16 = None
         # set by laenerf_b200.optim.ShardedFlatAdam: persistent fp32 gradient of the fp32 table, used when no autocast casts it
         self._grad_f32 = None
+        self._det_ws = DeterministicWorkspace()  # used only while torch.are_deterministic_algorithms_enabled()
 
     def reset_parameters(self):
         std = 1e-4
@@ -186,7 +222,7 @@ class GridEncoder(nn.Module):
         outputs = grid_encode(inputs, self.embeddings, self.offsets, self.per_level_scale, self.base_resolution,
                               inputs.requires_grad, self.gridtype_id, self.align_corners, self.interp_id,
                               shadow_f16(self, self.embeddings), self._grad_f16, float(bound) if in_kernel else 0.0, b_dev,
-                              self._grad_f32)
+                              self._grad_f32, self._det_ws)
         return outputs.view(prefix_shape + [self.output_dim])
 
     @torch.autocast(device_type="cuda", enabled=False)
@@ -200,6 +236,8 @@ class GridEncoder(nn.Module):
             B = inputs.shape[0]
         if self.embeddings.grad is None:
             raise ValueError("grad is None, should be called after loss.backward() and before optimizer.step()!")
+        # float atomics into the gradient, no deterministic kernel: raises (or warns under warn_only) as torch's own ops do
+        N.alert_not_deterministic("GridEncoder.grad_total_variation (lnrf_grad_total_variation)")
         inputs = inputs.contiguous().to(self.embeddings.dtype)
         N.check(N.lib().lnrf_grad_total_variation(N.ptr(inputs), N.ptr(self.embeddings), N.ptr(self.embeddings.grad),
                                                   N.ptr(_offsets_host(self.offsets)), float(weight), B, D, C, L, S, H,

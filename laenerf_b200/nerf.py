@@ -19,7 +19,7 @@ from torch.amp import custom_bwd, custom_fwd
 from . import _native as N
 from . import raymarching
 from ._shadow import half_of, shadow_f16
-from .ffmlp import FFMLP
+from .ffmlp import FFMLP, backward_deterministic
 from .gridencoder import GridEncoder
 from .shencoder import SHEncoder
 
@@ -141,6 +141,8 @@ class _fused_network(Function):
                 with torch.cuda.stream(N.defer_to_side_stream(dev)):
                     N.check(lib.lnrf_nerf_wgrad_reduce(N.ptr(scratch), nbytes, M, ns, nc, N.ptr(gws), N.ptr(gwc), 1, N.stream()))
         else:
+            if torch.are_deterministic_algorithms_enabled() and not backward_deterministic(32, 16, 64, ns, 0):
+                N.alert_not_deterministic(f"fused NeRF backward with a {ns}-layer sigma net (lnrf_nerf_backward, float-atomics weight gradient)")
             dh = torch.empty(M, 16, dtype=torch.half, device=dev)
             N.check(lib.lnrf_nerf_backward(N.ptr(grad_sigmas), N.ptr(grad_rgbs), N.ptr(rgbs), N.ptr(h0), N.ptr(enc), N.ptr(cin), N.ptr(ws),
                                            N.ptr(wc), N.ptr(fb), M, ns, nc, density_scale, N.ptr(grad_enc), N.ptr(gws), N.ptr(gwc),
@@ -173,7 +175,7 @@ class NeRFNetwork(nn.Module):
         self.register_buffer("density_bitfield", torch.zeros(self.cascade * grid_size ** 3 // 8, dtype=torch.uint8))
         self.register_buffer("step_counter", torch.zeros(16, 2, dtype=torch.int32))
         self._mean_host, self._mean_dev = 0.0, None  # behind the mean_density property
-        self._tmp_grid = self._occ_scratch = self._occ_mean = None
+        self._tmp_grid = self._occ_scratch = self._occ_mean = self._occ_winner = None
         self.iter_density = 0
         self.mean_count = 0
         self.local_step = 0
@@ -331,7 +333,12 @@ class NeRFNetwork(nn.Module):
             xyzs = torch.empty(n, 3, dtype=torch.float32, device=dev)
             N.check(lib.lnrf_occupancy_points(N.ptr(coords), N.ptr(u), n, H, float(bound_c), N.ptr(xyzs), N.ptr(indices), st))
             sig = self._density_scaled(xyzs).contiguous()
-            N.check(lib.lnrf_occupancy_scatter(N.ptr(sig), N.ptr(indices), n, N.ptr(tmp[cas]), st))
+            if torch.are_deterministic_algorithms_enabled():  # partial updates draw cells with repeats: the last occurrence wins
+                if self._occ_winner is None or self._occ_winner.device != dev:
+                    self._occ_winner = torch.full((H ** 3,), -1, dtype=torch.int32, device=dev)  # re-armed by the kernel
+                N.check(lib.lnrf_occupancy_scatter_det(N.ptr(sig), N.ptr(indices), n, N.ptr(tmp[cas]), N.ptr(self._occ_winner), H ** 3, st))
+            else:
+                N.check(lib.lnrf_occupancy_scatter(N.ptr(sig), N.ptr(indices), n, N.ptr(tmp[cas]), st))
         N.check(lib.lnrf_occupancy_ema(N.ptr(self.density_grid), N.ptr(tmp), self.density_grid.numel(), float(decay), float(self.density_thresh),
                                        N.ptr(self._occ_mean), N.ptr(self._occ_scratch), self._occ_scratch.numel() * 4, st))
         self._mean_dev = self._occ_mean
@@ -903,6 +910,13 @@ class TrainStep:
         self.scaler.update()
 
 
+def _check_mode(captured: bool, who: str) -> None:
+    """A graph replays the kernels of the mode it was captured in: never the other one silently."""
+    if captured != torch.are_deterministic_algorithms_enabled():
+        raise RuntimeError(f"{who}: captured with torch.are_deterministic_algorithms_enabled() == {captured}, but the flag is now "
+                           f"{not captured}; call capture() again (needs_recapture() reports the change)")
+
+
 class GraphedTrainStep:
     """The same training step replayed from ONE CUDA graph (march -> encode -> MLPs -> composite -> loss -> backward
     -> Adam): the 4096-ray step is launch-bound when issued from Python (SURVEY.md section 7, "hard parts"), so the
@@ -932,6 +946,7 @@ class GraphedTrainStep:
         self._pipe_opt = False
         self.sets = self.graphs = None  # lookahead: the two marched-batch buffer sets (with their targets) and the two graphs
         self.phase = 0                  # lookahead: the set the next replay trains on
+        self.deterministic = None       # torch.are_deterministic_algorithms_enabled() at capture: the graph holds that mode's kernels
 
     def _load(self, rays_o, rays_d, gt_rgb):
         self.ro.copy_(rays_o, non_blocking=True)
@@ -1018,19 +1033,23 @@ class GraphedTrainStep:
             with torch.cuda.graph(self.graph):
                 self.loss, self.out = self.step(self.ro, self.rd, self.gt, self.bg_color, self.perturb)
         self.captured_mean_count = m.mean_count
+        self.deterministic = torch.are_deterministic_algorithms_enabled()
         m.local_step = 0
         self._replays = 0
 
     def needs_recapture(self) -> bool:
-        """After update_mean_count(): re-capture when the running mean outgrew the captured buffer or shrank by > 1/8."""
+        """After update_mean_count(): re-capture when the running mean outgrew the captured buffer or shrank by > 1/8, or when
+        torch.use_deterministic_algorithms was switched since the capture."""
         mc, cap = self.model.mean_count, self.captured_mean_count
-        return self.graph is None or mc > cap or mc < cap - cap // 8
+        return (self.graph is None or mc > cap or mc < cap - cap // 8 or
+                self.deterministic != torch.are_deterministic_algorithms_enabled())
 
     def __call__(self, rays_o, rays_d, gt_rgb):
         if self.graph is None:
             self.capture(rays_o, rays_d, gt_rgb)
             if self.lookahead:  # the capture batch is in flight; its loss arrives with the next call
                 return None, None
+        _check_mode(self.deterministic, "GraphedTrainStep")
         self._load(rays_o, rays_d, gt_rgb)
         m = self.model
         if m.render_clip_far:

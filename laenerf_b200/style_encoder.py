@@ -242,6 +242,11 @@ class GraphedStyleTrainStep:
         self.t = torch.zeros(n_points, 3, device=dev)
         self.graph = None
         self.loss = self.pred = None
+        self.deterministic = None  # torch.are_deterministic_algorithms_enabled() at capture
+
+    def needs_recapture(self) -> bool:
+        """True before the first capture and after torch.use_deterministic_algorithms was switched since the capture."""
+        return self.graph is None or self.deterministic != torch.are_deterministic_algorithms_enabled()
 
     def capture(self, x_term, d, target, warmup: int = 3):
         self.x.copy_(x_term); self.d.copy_(d); self.t.copy_(target)
@@ -254,10 +259,13 @@ class GraphedStyleTrainStep:
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph):
             self.loss, self.pred = self.step(self.x, self.d, self.t)
+        self.deterministic = torch.are_deterministic_algorithms_enabled()
 
     def __call__(self, x_term, d, target):
         if self.graph is None:
             self.capture(x_term, d, target)
+        from .nerf import _check_mode
+        _check_mode(self.deterministic, "GraphedStyleTrainStep")
         self.x.copy_(x_term, non_blocking=True); self.d.copy_(d, non_blocking=True); self.t.copy_(target, non_blocking=True)
         self.graph.replay()
         self.step.style_step += 1
